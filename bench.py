@@ -38,6 +38,13 @@ METRIC = "env-steps/s (layered obs, device-timed)"
 UNIT = "env-steps/s"
 # bounded timed steps of the other configs: (steps, warm-up) — about 0.1-0.2 s of device time each
 CONFIG_STEPS = {1: (512, 16), 3: (96, 8), 4: (32, 4), 5: (8, 3)}
+# steps from the reset at creation to the state the timed steps start from: an episode of level 6 under random actions lasts
+# about 20 steps, so by then the batch has the mix of running and resetting envs of a long-running job
+SETTLE_STEPS = 256
+# --dump-outputs: at most this many bytes of float32 rows; above it, a fixed seeded sample of the envs is written
+DUMP_BYTES = 64 << 20
+DUMP_SEED = 7
+OUTPUTS = ("obs", "state", "avail", "reward", "done", "events", "actions", "err")
 
 
 def level_text(n: int) -> str:
@@ -167,6 +174,24 @@ def run_reference(args) -> None:
     print(json.dumps(line))
 
 
+def output_rows(vec, begin: int, n_total: int) -> dict:
+    """This rank's rows of what the last step handed its caller (the per-env output tensors of VecWorld), as float32 numpy arrays,
+    plus their global env ids as float64.  All envs when their rows fit in DUMP_BYTES, else a fixed seeded sample of the global
+    env ids, the same for every rank count."""
+    import numpy as np
+    import torch
+
+    tensors = {name: getattr(vec, name) for name in OUTPUTS}
+    row_bytes = 8 + sum(4 * t[0].numel() for t in tensors.values())
+    n_keep = min(n_total, DUMP_BYTES // row_bytes)
+    ids = np.arange(n_total) if n_keep == n_total else np.sort(np.random.default_rng(DUMP_SEED).choice(n_total, n_keep, replace=False))
+    ids = ids[(ids >= begin) & (ids < begin + vec.n_envs)]
+    rows = torch.from_numpy(ids - begin).to(vec.device)
+    out = {name: t.index_select(0, rows).float().cpu().numpy() for name, t in tensors.items()}
+    out["env_id"] = ids.astype(np.float64)
+    return out
+
+
 def pin_rank_to_cores(local_rank: int, local_world: int) -> list[int] | None:
     """One disjoint slice of the host cores per rank: the step loop of a rank is host-driven (one launch per step), and
     eight Python processes migrating over the same cores show up as per-rank jitter in the MAX-over-ranks timing."""
@@ -236,7 +261,12 @@ def run_ours(args) -> None:
 
     # ---------------- device-resident arm: K fused steps back to back, no host sync inside.
     # Untimed preheat first (not counted as warm-up steps): a fresh process finds the GPU at idle clocks, and W = 5 steps are
-    # 0.4 ms of work; the timed window should see the clocks a running job sees.
+    # 0.4 ms of work; the timed window should see the clocks a running job sees.  The preheat runs for a wall-clock time, so
+    # its number of steps varies: the state after SETTLE_STEPS is restored after it, and every run with the same arguments
+    # times the same steps on the same inputs.
+    for _ in range(SETTLE_STEPS):
+        vec.step(None)
+    settled = vec.checkpoint()
     sampler = ClockSampler(local_rank) if rank == 0 else None
     t0 = time.perf_counter()
     preheat = 0
@@ -250,6 +280,8 @@ def run_ours(args) -> None:
             vec.step(None)
         preheat += 64
         torch.cuda.synchronize()
+    vec.restore(settled)
+    del settled
     for _ in range(Wm):
         vec.step(None)
     barrier()
@@ -260,6 +292,13 @@ def run_ours(args) -> None:
     ms_total, timed_launches = vec.timing_end()
     barrier()
     launches = vec.launch_count - launches0
+    dumped = None
+    if args.dump_outputs:
+        dumped = output_rows(vec, begin, args.envs * world_size)
+        if world_size > 1:
+            parts = [None] * world_size
+            dist.all_gather_object(parts, dumped)
+            dumped = {name: np.concatenate([p[name] for p in parts]) for name in dumped}
     per_rank = gather(ms_total / K)
     ms_max = max(per_rank) * K
     value = world_size * n_envs * K / (ms_max / 1e3)
@@ -497,6 +536,10 @@ def run_ours(args) -> None:
             cb = cpu_baseline()
             cb.pop("seconds", None)
             line["cpu_baseline"] = cb
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumped.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
         print(json.dumps(line))
     if world_size > 1:
         dist.destroy_process_group()
@@ -517,7 +560,13 @@ def main():
     ap.add_argument("--no-compiled-host", action="store_true", help="skip the compiled-host closed loop of the e2e arm")
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE workloads")
     ap.add_argument("--no-closed-loop", action="store_true", help="skip the closed loop over parts (implied under ncu, which serialises launches)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (float32; "
+                    "env_id.npy: the envs the rows belong to, a fixed sample when all envs would exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -348,10 +348,29 @@ def main():
                     break
                 store(arrays, index, name, text, cfg, policy, rec)
         print(name, "done", file=sys.stderr)
-    arrays["index"] = np.frombuffer(json.dumps(index).encode(), dtype=np.uint8)
     out = os.path.join(HERE, "env_vectors.npz")
-    np.savez_compressed(out, **arrays)
+    save(arrays, index, out)
     print(f"{out}: {len(index)} cases, {os.path.getsize(out) / 1e6:.2f} MB")
+
+
+def save(arrays: dict, index: list, out: str) -> None:
+    """One flat array per dtype, a JSON layout (key -> dtype, offset, shape) and the JSON index, in an .npz whose entries are
+    LZMA-compressed: two thousand small entries cost more in zip headers than in data, and LZMA packs the observations several
+    times tighter than deflate.  tests/test_env_vectors.py cuts the arrays back out of the flat ones."""
+    import zipfile
+
+    flat, layout = {}, {}
+    for key, a in arrays.items():
+        parts = flat.setdefault(a.dtype.name, [])
+        layout[key] = [a.dtype.name, sum(p.size for p in parts), list(a.shape)]
+        parts.append(a.ravel())
+    entries = {name: np.concatenate(parts) for name, parts in flat.items()}
+    entries["layout"] = np.frombuffer(json.dumps(layout).encode(), dtype=np.uint8)
+    entries["index"] = np.frombuffer(json.dumps(index).encode(), dtype=np.uint8)
+    with zipfile.ZipFile(out, "w", compression=zipfile.ZIP_LZMA) as zf:
+        for name, a in entries.items():
+            with zf.open(name + ".npy", "w", force_zip64=True) as f:
+                np.lib.format.write_array(f, a)
 
 
 if __name__ == "__main__":

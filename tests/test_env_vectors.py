@@ -22,7 +22,11 @@ def data():
     global _DATA
     if _DATA is None:
         z = np.load(os.path.join(GOLDEN, "env_vectors.npz"))
-        _DATA = (z, json.loads(bytes(z["index"]).decode()))
+        # the file holds one flat array per dtype (tests/golden/make_env_vectors.py: save); the layout cuts the recorded arrays out
+        layout = json.loads(bytes(z["layout"]).decode())
+        flat = {dt: z[dt] for dt in {dt for dt, _, _ in layout.values()}}
+        arrays = {key: flat[dt][off:off + int(np.prod(shape))].reshape(shape) for key, (dt, off, shape) in layout.items()}
+        _DATA = (arrays, json.loads(bytes(z["index"]).decode()))
     return _DATA
 
 
@@ -51,7 +55,7 @@ def replay(api, entry, obs_type, check_env=True):
     want_obs = z[f"{key}|obs|{obs_type}"]
     tiled = entry["obs_tiled"][obs_type]
     avail, extras, state = z[f"{key}|avail"], z[f"{key}|extras"], z[f"{key}|state"]
-    reward = z[f"{key}|reward"] if f"{key}|reward" in z.files else None
+    reward = z[f"{key}|reward"] if f"{key}|reward" in z else None
     n_step = 0
     for row, op in enumerate(entry["script"]):
         where = f"{key} [{obs_type}] op {row} ({op['op']})"
