@@ -165,6 +165,17 @@ __device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_
     uint32_t s = (uint32_t)__cvta_generic_to_shared(ssrc);
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(s), "r"(bytes) : "memory");
 }
+// The same with an L2 eviction policy (createpolicy): observation rows are written once per step and not read by the kernel
+__device__ __forceinline__ void bulk_store_hint(void* gdst, const void* ssrc, uint32_t bytes, uint64_t policy) {
+    uint32_t s = (uint32_t)__cvta_generic_to_shared(ssrc);
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(gdst), "r"(s), "r"(bytes), "l"(policy)
+                 : "memory");
+}
+__device__ __forceinline__ uint64_t l2_evict_first_policy() {
+    uint64_t policy;
+    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(policy));
+    return policy;
+}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
@@ -1278,7 +1289,10 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                 fence_proxy_async_smem();  // generic-proxy writes above -> visible to the async proxy
                 __syncwarp();
                 if (lane == 0) {
-                    bulk_store(p.obs + (env0 + (int64_t)tix * p.E) * p.obs_stride, tiles, (uint32_t)(p.E * p.obs_stride) * 4u);
+                    // evict-first: the rows stream through L2 to HBM (491 MB per level-6 step of 65,536 worlds, four times the L2)
+                    // and should not push out the records, flags and small outputs the next step reads and rewrites
+                    bulk_store_hint(p.obs + (env0 + (int64_t)tix * p.E) * p.obs_stride, tiles, (uint32_t)(p.E * p.obs_stride) * 4u,
+                                    l2_evict_first_policy());
                     bulk_commit();
                     if (p.timeline) {
                         t_last = globaltimer_ns();
