@@ -160,8 +160,13 @@ typedef struct {
     /* 1: also keep, per env, Step.info of LLE.step (python/lle/env/env.py:174-188) and episode statistics, written by the step kernel
      * (lle_vec_buffers.info / ep_return / ep_length / last_return / last_length): about 20 more bytes per env-step. */
     int32_t episode_stats;
+    /* Element type of `obs` (LLE_DTYPE_*).  Every value of a layered, padded, flattened or perspective observation is -1, 0 or 1,
+     * so LLE_DTYPE_I8 stores the same observation in a quarter of the bytes (lle_vec_buffers.obs_i8; `obs` is then NULL).
+     * LLE_OBS_PARTIAL and LLE_OBS_STATE are f32 only.  The state_type observation (state_obs) is always f32. */
+    int32_t obs_dtype;
 } lle_vec_options;
 enum { LLE_OBS_LAYERED = 0, LLE_OBS_PARTIAL = 1, LLE_OBS_PERSPECTIVE = 2, LLE_OBS_STATE = 3 };
+enum { LLE_DTYPE_F32 = 0, LLE_DTYPE_I8 = 1 };
 LLE_API void lle_vec_default_options(lle_vec_options* opts);
 
 /* All maps must share (height, width, n_agents, n_gems).  map_of_env may be NULL (every env uses maps[0]). */
@@ -171,6 +176,7 @@ LLE_API int lle_vec_destroy(lle_vec* vec);
 
 /* Device pointers of the per-step outputs (valid until lle_vec_destroy).  Layouts, C-contiguous:
  *   obs      f32 [N, obs_stride]   one block per env (obs_stride = block length rounded up to 4 floats), by obs_type:
+ *            (obs_i8: i8 [N, obs_stride] instead, obs_stride rounded up to 16 bytes, when obs_dtype is LLE_DTYPE_I8)
  *                                    layered      (C,H,W) = LayeredPadded.observe()[0] (observations.py:254-266), C = 2(A+padding)+4;
  *                                                 the reference's (A+padding,C,H,W) np.tile is a stride-0 repeat of it
  *                                    partial      (A, 2A+3, size, size): every agent's own window (:331-350)
@@ -189,7 +195,7 @@ LLE_API int lle_vec_destroy(lle_vec* vec);
 typedef struct {
     int64_t n_envs;
     int32_t n_agents, n_gems, n_channels, height, width, reward_dim, state_dim, n_beams_max;
-    int64_t obs_stride; /* floats */
+    int64_t obs_stride; /* elements of the vec's obs_dtype: a multiple of 4 (f32) or of 16 (i8) */
     float* obs;
     float* state;
     uint8_t* avail;
@@ -227,6 +233,10 @@ typedef struct {
     int32_t* ep_length;
     float* last_return;
     int32_t* last_length;
+    /* obs_dtype LLE_DTYPE_I8: the observation rows (obs is NULL); NULL for an f32 vec */
+    int8_t* obs_i8;
+    int32_t obs_dtype;
+    int32_t pad4;
 } lle_vec_buffers;
 LLE_API int lle_vec_get_buffers(lle_vec* vec, lle_vec_buffers* out);
 

@@ -40,7 +40,7 @@ class VecOptions(C.Structure):
         ("seed", C.c_uint64), ("env_id_base", C.c_uint64), ("n_extras", C.c_int32), ("extras_src", C.c_int32 * 64),
         ("pbrs", C.c_int32), ("n_pbrs", C.c_int32), ("pbrs_src", C.c_int32 * 64), ("pbrs_gamma", C.c_double),
         ("pbrs_reward_value", C.c_double), ("obs_type", C.c_int32), ("obs_param", C.c_int32), ("randomize_lasers", C.c_int32),
-        ("state_type", C.c_int32), ("state_param", C.c_int32), ("episode_stats", C.c_int32)]
+        ("state_type", C.c_int32), ("state_param", C.c_int32), ("episode_stats", C.c_int32), ("obs_dtype", C.c_int32)]
 
 
 class VecBuffers(C.Structure):
@@ -51,7 +51,11 @@ class VecBuffers(C.Structure):
         (n, C.c_int32) for n in ("obs_type", "obs_param", "obs_view_agents", "obs_c", "obs_h", "obs_w", "obs_invalid", "pad2")] + [
         ("map_index", C.c_void_p), ("n_variants", C.c_int32), ("pad3", C.c_int32), ("state_obs", C.c_void_p), ("state_obs_stride", C.c_int64)] + [
         (n, C.c_int32) for n in ("state_type", "state_param", "state_view_agents", "state_c", "state_h", "state_w")] + [
-        (n, C.c_void_p) for n in ("info", "ep_return", "ep_length", "last_return", "last_length")]
+        (n, C.c_void_p) for n in ("info", "ep_return", "ep_length", "last_return", "last_length")] + [
+        ("obs_i8", C.c_void_p), ("obs_dtype", C.c_int32), ("pad4", C.c_int32)]
+
+# lle_vec_options.obs_dtype
+DTYPE_F32, DTYPE_I8 = 0, 1
 
 
 class RawState(C.Structure):

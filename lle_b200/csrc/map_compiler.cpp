@@ -423,7 +423,16 @@ CompiledMap compile_map(const std::string& text, const ObsSpec& spec, const std:
     h.cellbeams_off = (uint32_t)off; off = align16(off + (size_t)HW * sizeof(LleCellBeams));
     h.beams_off = (uint32_t)off;   off = align16(off + (size_t)std::max(NB, 1) * sizeof(LleBeam));
     h.patch_off = (uint32_t)off;   off = align16(off + std::max<size_t>(patch.size(), 1) * sizeof(LlePatch));
-    h.static_off = (uint32_t)off;  off = align16(off + stat.size() * sizeof(float));
+    // An int8 observation (obs_dtype) takes its static plane as bytes, zero-padded to the row stride (a multiple of 16): every
+    // 16-byte piece of a row is then one asynchronous copy from the plane.
+    const bool i8 = spec.dtype == LLE_DTYPE_I8;
+    std::vector<int8_t> stat_i8;
+    if (i8) {
+        stat_i8.assign(((size_t)obs_floats + 15) / 16 * 16, 0);
+        for (size_t k = 0; k < stat.size() && k < stat_i8.size(); ++k) stat_i8[k] = (int8_t)stat[k];
+    }
+    h.obs_dtype = spec.dtype;
+    h.static_off = (uint32_t)off;  off = align16(off + (i8 ? stat_i8.size() : stat.size() * sizeof(float)));
     h.ap_off = (uint32_t)off;      off = align16(off + std::max<size_t>(planes.size(), 1) * sizeof(LleAgentPlane));
     h.n_static = n_static;
     h.static_list_off = (uint32_t)off; off = align16(off + std::max<size_t>(static_list.size(), 1) * sizeof(LlePatch));
@@ -441,8 +450,10 @@ CompiledMap compile_map(const std::string& text, const ObsSpec& spec, const std:
     for (int a = 0; a < A; ++a) h.start_order[a] = (uint8_t)order[a];
     std::vector<uint32_t> chunk_tbl;  // patches are sorted by idx: chunk c owns entries [tbl[c], tbl[c+1])
     {
-        const int64_t block = ((int64_t)obs_floats + 3) / 4 * 4;  // the vec pads a block to 4 floats (obs_stride)
-        const int chunk = lle_chunk_floats(block);
+        // the vec pads a block to 16 bytes (obs_stride): 4 floats or 16 int8 elements
+        const int per16 = i8 ? 16 : 4;
+        const int64_t block = ((int64_t)obs_floats + per16 - 1) / per16 * per16;
+        const int chunk = lle_chunk_elems(block, i8 ? 1 : 4);
         const int n_chunks = (int)((block + chunk - 1) / chunk);
         size_t k = 0;
         for (int c = 0; c <= n_chunks; ++c) {
@@ -513,7 +524,8 @@ CompiledMap compile_map(const std::string& text, const ObsSpec& spec, const std:
     }
     if (!patch.empty()) std::memcpy(cm.blob.data() + h.patch_off, patch.data(), patch.size() * sizeof(LlePatch));
     if (!static_list.empty()) std::memcpy(cm.blob.data() + h.static_list_off, static_list.data(), static_list.size() * sizeof(LlePatch));
-    std::memcpy(cm.blob.data() + h.static_off, stat.data(), stat.size() * sizeof(float));
+    if (i8) std::memcpy(cm.blob.data() + h.static_off, stat_i8.data(), stat_i8.size());
+    else std::memcpy(cm.blob.data() + h.static_off, stat.data(), stat.size() * sizeof(float));
     std::memcpy(cm.blob.data() + h.chunk_tbl_off, chunk_tbl.data(), chunk_tbl.size() * sizeof(uint32_t));
     std::memcpy(cm.blob.data() + h.cand_index_off, cand_index.data(), cand_index.size() * sizeof(uint32_t));
     if (!cand_pos.empty()) std::memcpy(cm.blob.data() + h.cand_pos_off, cand_pos.data(), cand_pos.size() * sizeof(uint16_t));

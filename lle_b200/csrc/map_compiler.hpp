@@ -75,7 +75,8 @@ struct CompiledMap {
 struct ObsSpec {
     int kind = LLE_OBS_LAYERED;
     int param = 0;
-    bool operator==(const ObsSpec& o) const { return kind == o.kind && param == o.param; }
+    int dtype = LLE_DTYPE_F32;  // element type of the static plane (LLE_DTYPE_I8: int8_t, for layered / perspective only)
+    bool operator==(const ObsSpec& o) const { return kind == o.kind && param == o.param && dtype == o.dtype; }
 };
 
 // State of a laser source after the world was built: LaserBeam::{set_agent_id, enable, disable} (src/core/tiles/laser.rs:69-84).

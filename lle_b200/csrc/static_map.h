@@ -75,13 +75,16 @@ struct LleAgentPlane {
 // boundaries split a line between two bulk stores, measured 6 % slower than 3,072).
 // Only done when the last 3,072-float chunk would be less than half full (on a 64x64 map, 26 x 12 KB + 8 KB, equal
 // chunks of 3,040 floats were 1 % slower).
-static inline int lle_chunk_floats(int64_t block_floats) {
-    const int64_t rest = block_floats % LLE_CHUNK_FLOATS;
-    if (rest == 0 || rest >= LLE_CHUNK_FLOATS / 2) return LLE_CHUNK_FLOATS;
-    const int64_t n = (block_floats + LLE_CHUNK_FLOATS - 1) / LLE_CHUNK_FLOATS;
-    const int64_t len = (block_floats + n - 1) / n;
-    return (int)((len + 31) / 32 * 32);
+// An int8 block is cut by the same byte budget: chunks of up to 12,288 elements on 128-byte lines.
+static inline int lle_chunk_elems(int64_t block, int elem_bytes) {
+    const int64_t max_len = LLE_CHUNK_FLOATS * 4 / elem_bytes, line = 128 / elem_bytes;
+    const int64_t rest = block % max_len;
+    if (rest == 0 || rest >= max_len / 2) return (int)max_len;
+    const int64_t n = (block + max_len - 1) / max_len;
+    const int64_t len = (block + n - 1) / n;
+    return (int)((len + line - 1) / line * line);
 }
+static inline int lle_chunk_floats(int64_t block_floats) { return lle_chunk_elems(block_floats, 4); }
 #endif
 struct LleCellBeams {
     uint32_t e[4];
@@ -91,13 +94,13 @@ struct LleCellBeams {
 struct LleMapHeader {
     int32_t H, W, A, G, NB, C;
     int32_t n_patch;
-    int32_t obs_floats;       // C*H*W
+    int32_t obs_floats;       // C*H*W (elements, whatever the element type)
     uint32_t tiles_off;       // uint16_t[H*W]
     uint32_t cellinfo_off;    // uint32_t[H*W]
     uint32_t cellbeams_off;   // LleCellBeams[H*W]
     uint32_t beams_off;       // LleBeam[NB]
     uint32_t patch_off;       // LlePatch[n_patch]
-    uint32_t static_off;      // float[C*H*W]
+    uint32_t static_off;      // float[C*H*W], or int8_t[C*H*W rounded up to 16] for an int8 observation (obs_dtype)
     uint32_t blob_bytes;
     uint32_t obs_invalid;     // some LASER_0+colour >= C: the reference raises IndexError (observations.py:235)
     uint64_t gem_toplevel;    // bit g set <=> gem g is NOT wrapped by a laser (world.rs:265-275, :550-554)
@@ -106,7 +109,7 @@ struct LleMapHeader {
     int32_t obs_c, obs_h, obs_w;   // shape of ONE agent's observation (state: obs_c = length, obs_h = obs_w = 0)
     int32_t n_ap;                  // entries of the agent-plane table
     uint32_t ap_off;               // LleAgentPlane[n_ap]
-    uint32_t chunk_tbl_off;        // uint32_t[n_chunks + 1]: patch index range of every chunk of lle_chunk_floats(padded block) floats
+    uint32_t chunk_tbl_off;        // uint32_t[n_chunks + 1]: patch index range of every chunk of lle_chunk_elems(padded block) elements
     int32_t n_static;              // layered observations: non-zero floats of the static plane, listed at static_list_off
     int32_t random_starts;         // some agent has several start candidates: World::reset samples (world.rs:421)
     uint32_t cand_index_off;       // uint32_t[2*A]: first index and count of each agent's candidates in cand_pos
@@ -115,6 +118,8 @@ struct LleMapHeader {
     uint8_t start_order[LLE_MAX_AGENTS];  // agents by increasing number of candidates (stable), the order sample_different assigns them
     uint16_t start[LLE_MAX_AGENTS];   // packed position (i<<8 | j); with random starts: the first candidate
     uint16_t gem_pos[LLE_MAX_GEMS];   // packed position, gems_positions order (parser_v1.rs:149)
+    int32_t obs_dtype;                // LLE_DTYPE_*: element type of the static plane and of the observation rows
+    int32_t pad_dtype;
 };
 
 // ---- dynamic per-env record: `stride` 32-bit words per environment, stored contiguously (array of

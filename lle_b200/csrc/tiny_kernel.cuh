@@ -62,7 +62,9 @@ __device__ __forceinline__ void store_bytes(uint8_t* dst, const uint32_t (&b)[N]
 
 // PARTIAL: the observation is PartialGenerator's (A windows of size x size per world, tiny_core.cuh partial_cell_task) instead of
 // the layered block; its own instantiation, so that the layered kernel keeps its 72 registers / 7 CTAs per SM.
-template <int A_, bool PARTIAL = false>
+// OT: the observation's element type, float or int8_t (lle_vec_options.obs_dtype; PARTIAL is float only).  An int8 tile is
+// zero-filled and drawn in bytes and leaves with a bulk store of a quarter of the size.
+template <int A_, bool PARTIAL = false, typename OT = float>
 __global__ void __launch_bounds__(kThreads, PARTIAL ? 4 : LLE_TINY_MIN_CTAS) lle_tiny_step_kernel(const KParams p) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -74,7 +76,7 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 4 : LLE_TINY_MIN_CTAS) lle
     uint32_t* snext = srec + stride * 32;                                            // [32][stride]: the NEXT ticket's records, prefetched
     const LlePatch** slptr = reinterpret_cast<const LlePatch**>(snext + stride * 32); // [32]: the render list of lane l's map (PARTIAL: its cellinfo)
     uint32_t* smeta = reinterpret_cast<uint32_t*>(slptr + 32);                       // [32]: n_static | n_patch << 16 of lane l's map
-    float* tile = reinterpret_cast<float*>(smeta + 32 + (PARTIAL ? 64 : 0));         // [E][ostr]: E worlds per bulk store
+    OT* tile = reinterpret_cast<OT*>(smeta + 32 + (PARTIAL ? 64 : 0));               // [E][ostr]: E worlds per bulk store
     const LleCellBeams** sbeams = reinterpret_cast<const LleCellBeams**>(smeta + 32);  // PARTIAL: [32] the beam table of lane l's map
     const int E = p.E;
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
@@ -301,10 +303,13 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 4 : LLE_TINY_MIN_CTAS) lle
                 // warps per SM, and even the unused run-time branch for it cost 3 %.)
                 if (lane == 0) bulk_wait_read<0>();
                 __syncwarp();
-                for (int f = lane * 4; f < E * ostr; f += 128) *reinterpret_cast<float4*>(tile + f) = make_float4(0.f, 0.f, 0.f, 0.f);
+                if constexpr (sizeof(OT) == 4)
+                    for (int f = lane * 4; f < E * ostr; f += 128) *reinterpret_cast<float4*>(tile + f) = make_float4(0.f, 0.f, 0.f, 0.f);
+                else
+                    for (int f = lane * 16; f < E * ostr; f += 512) *reinterpret_cast<uint4*>(tile + f) = make_uint4(0u, 0u, 0u, 0u);
                 __syncwarp();
                 const int ws = (r << lgE) + (lane >> lgl), q = lane & (lpw - 1);  // the world this lane helps to draw, and its share
-                float* sub = tile + (size_t)(lane >> lgl) * ostr;
+                OT* sub = tile + (size_t)(lane >> lgl) * ostr;
                 auto agent_pos = [&](int a) {
                     const uint32_t wd = srec[(a >> 1) * 32 + ws];
                     return (a & 1) ? (wd >> 16) : (wd & 0xFFFFu);
@@ -325,10 +330,10 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 4 : LLE_TINY_MIN_CTAS) lle
                     const int ns = (int)(meta & 0xFFFFu), n = ns + (int)(meta >> 16);
                     auto draw = [&](const LlePatch pe, int k) {
                         if (k < ns) {
-                            sub[pe.idx] = (float)pe.stat;  // static layers (observations.py:216-237)
+                            sub[pe.idx] = (OT)pe.stat;  // static layers (observations.py:216-237)
                         } else {
                             const uint32_t wd = srec[(pe.src == 0xFF ? w_gems : w_on + pe.src) * 32 + ws];
-                            if ((((wd >> pe.bit) & 1u) != 0) != (pe.src == 0xFF)) sub[pe.idx] = 1.0f;  // lit laser cell / uncollected gem (:256-263)
+                            if ((((wd >> pe.bit) & 1u) != 0) != (pe.src == 0xFF)) sub[pe.idx] = (OT)1;  // lit laser cell / uncollected gem (:256-263)
                         }
                     };
                     const LlePatch* list = slptr[ws];
@@ -346,13 +351,13 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 4 : LLE_TINY_MIN_CTAS) lle
 #endif
                     for (int a = q; a < A_; a += lpw) {  // the agents' one-hots (:264-265): their planes hold nothing else
                         const uint32_t pp = agent_pos(a);
-                        sub[a * p.HW + (int)(pp >> 8) * W + (int)(pp & 0xFFu)] = 1.0f;
+                        sub[a * p.HW + (int)(pp >> 8) * W + (int)(pp & 0xFFu)] = (OT)1;
                     }
                 }
                 fence_proxy_async_smem();
                 __syncwarp();
                 if (lane == 0) {
-                    bulk_store(p.obs + ((int64_t)ticket * 32 + ((int64_t)r << lgE)) * ostr, tile, (uint32_t)(E * ostr) * 4u);
+                    bulk_store(obs_rows<OT>(p) + ((int64_t)ticket * 32 + ((int64_t)r << lgE)) * ostr, tile, (uint32_t)(E * ostr) * (uint32_t)sizeof(OT));
                     bulk_commit();
                     if (owed && r == 0) {
                         bulk_wait<1>();  // every store but the one just issued has completed: the previous ticket is done

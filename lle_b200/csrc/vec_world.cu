@@ -71,6 +71,8 @@ struct lle_vec {
     int32_t* d_map_of_env = nullptr;
     uint32_t* d_records = nullptr;
     float* d_obs = nullptr;
+    int8_t* d_obs_i8 = nullptr;  // obs_dtype LLE_DTYPE_I8: the observation rows (d_obs stays null)
+    bool i8 = false;             // the observation is rendered in int8 (the kernels' OT = int8_t)
     float* d_state = nullptr;
     uint8_t* d_avail = nullptr;
     float* d_reward = nullptr;
@@ -153,6 +155,46 @@ namespace {
 constexpr int kSchedSlots = 8;
 constexpr int kSchedSlotWords = 32;
 
+// The thread-per-world step kernel of a vec with A agents (tiny_kernel.cuh): one instantiation per agent count and element type
+template <typename OT>
+cudaError_t launch_tiny(const lle_vec* v, const cudaLaunchConfig_t& cfg, const KParams& p) {
+    if constexpr (sizeof(OT) == 4) {
+        switch (v->A * 2 + (v->tiny_partial ? 1 : 0)) {
+            case 2: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<1, false>, p);
+            case 3: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<1, true>, p);
+            case 4: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<2, false>, p);
+            case 5: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<2, true>, p);
+            case 6: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<3, false>, p);
+            case 7: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<3, true>, p);
+            case 8: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<4, false>, p);
+            default: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<4, true>, p);
+        }
+    } else {  // partial observations are float only
+        switch (v->A) {
+            case 1: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<1, false, OT>, p);
+            case 2: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<2, false, OT>, p);
+            case 3: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<3, false, OT>, p);
+            default: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<4, false, OT>, p);
+        }
+    }
+}
+
+template <int MODE, typename OT>
+cudaError_t launch_world(const lle_vec* v, const cudaLaunchConfig_t& cfg, const KParams& p) {
+    if constexpr (MODE == MODE_STEP) {
+        if (p.part_in) {  // a parts loop: its own instantiations
+            if (v->fast) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 1, true, OT>, p);
+            if constexpr (sizeof(OT) == 4)
+                if (v->by_feature) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 2, true>, p);
+            return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 0, true, OT>, p);
+        }
+    }
+    if (v->fast) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 1, false, OT>, p);
+    if constexpr (sizeof(OT) == 4)  // the feature-driven renderer draws partial observations: float only
+        if (v->by_feature) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 2>, p);
+    return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 0, false, OT>, p);
+}
+
 template <int MODE>
 cudaError_t launch_mode(lle_vec* v, KParams& p, cudaStream_t s) {
     // Programmatic stream serialization: the kernel calls griddepcontrol.wait before it touches anything a
@@ -190,28 +232,10 @@ cudaError_t launch_mode(lle_vec* v, KParams& p, cudaStream_t s) {
             p.tile_floats = (int32_t)(v->tiny_E * v->obs_stride);
             p.warp_smem_bytes = v->tiny_warp_smem;
             p.ticket_chunk = v->tiny_chunk;
-            switch (v->A * 2 + (v->tiny_partial ? 1 : 0)) {
-                case 2: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<1, false>, p);
-                case 3: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<1, true>, p);
-                case 4: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<2, false>, p);
-                case 5: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<2, true>, p);
-                case 6: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<3, false>, p);
-                case 7: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<3, true>, p);
-                case 8: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<4, false>, p);
-                default: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<4, true>, p);
-            }
+            return v->i8 ? launch_tiny<int8_t>(v, cfg, p) : launch_tiny<float>(v, cfg, p);
         }
     }
-    if constexpr (MODE == MODE_STEP) {
-        if (p.part_in) {  // a parts loop: its own instantiations
-            if (v->fast) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 1, true>, p);
-            if (v->by_feature) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 2, true>, p);
-            return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 0, true>, p);
-        }
-    }
-    if (v->fast) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 1>, p);
-    if (v->by_feature) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 2>, p);
-    return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 0>, p);
+    return v->i8 ? launch_world<MODE, int8_t>(v, cfg, p) : launch_world<MODE, float>(v, cfg, p);
 }
 // Host bookkeeping (launch index, sequence number, "the last launch was a step") advances only when the launch was accepted.
 cudaError_t launch(lle_vec* v, KParams& p, cudaStream_t s) {
@@ -285,9 +309,9 @@ cudaError_t smem_optin(int device, int* out) {
     return cudaSuccess;
 }
 
-template <int MODE, int KIND, bool PARTS = false>
+template <int MODE, int KIND, bool PARTS = false, typename OT = float>
 cudaError_t configure_kernel(size_t smem, int* blocks) {
-    auto kern = lle_world_kernel<MODE, KIND, PARTS>;
+    auto kern = lle_world_kernel<MODE, KIND, PARTS, OT>;
     int dev = 0, optin = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = smem_optin(dev, &optin);
@@ -336,7 +360,7 @@ KParams base_params(lle_vec* v) {
     p.N_pad = v->N_pad;
     p.A = v->A; p.G = v->G; p.NBmax = v->NBmax; p.C = v->C; p.H = v->H; p.W = v->W; p.S = v->S; p.R = v->R;
     p.HW = v->H * v->W;
-    p.obs = v->d_obs; p.obs_stride = v->obs_stride;
+    p.obs = v->d_obs; p.obs_i8 = v->d_obs_i8; p.obs_stride = v->obs_stride;
     p.state = v->d_state; p.avail = v->d_avail; p.reward = v->d_reward; p.done = v->d_done;
     p.events = v->d_events; p.actions = v->d_actions; p.err = v->d_err;
     p.seed = v->opts.seed; p.env_id_base = v->opts.env_id_base; p.t = v->t;
@@ -515,6 +539,7 @@ void lle_vec_default_options(lle_vec_options* o) {
     o->seed = 0; o->env_id_base = 0;
     o->n_extras = 0; o->pbrs = 0; o->n_pbrs = -1; o->pbrs_gamma = 0.99; o->pbrs_reward_value = 0.5;  // Builder.pbrs defaults (builder.py:79-80)
     o->state_type = LLE_OBS_STATE; o->state_param = 0;  // ObservationType.STATE (builder.py:22)
+    o->obs_dtype = LLE_DTYPE_F32;
 }
 
 int lle_vec_destroy(lle_vec* v) {
@@ -525,7 +550,7 @@ int lle_vec_destroy(lle_vec* v) {
     if (v->borrows_records) { v->d_records = nullptr; v->d_map_of_env = nullptr; }
     for (auto* b : v->d_blobs) cudaFree(b);
     for (auto* b : v->retired_blobs) cudaFree(b);
-    cudaFree((void*)v->d_blob_table); cudaFree(v->d_map_of_env); cudaFree(v->d_records); cudaFree(v->d_obs); cudaFree(v->d_state);
+    cudaFree((void*)v->d_blob_table); cudaFree(v->d_map_of_env); cudaFree(v->d_records); cudaFree(v->d_obs); cudaFree(v->d_obs_i8); cudaFree(v->d_state);
     cudaFree(v->d_avail); cudaFree(v->d_reward); cudaFree(v->d_done); cudaFree(v->d_events); cudaFree(v->d_actions);
     cudaFree(v->d_err); cudaFree(v->d_sched); cudaFree(v->d_flags); cudaFree(v->d_actions_stage); cudaFree(v->d_timeline); cudaFree(v->d_extras);
     cudaFree(v->d_info); cudaFree(v->d_ep_return); cudaFree(v->d_last_return); cudaFree(v->d_ep_length); cudaFree(v->d_last_length);
@@ -552,12 +577,17 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
                    const lle_vec_options* opts, lle_vec** out) {
     if (!maps || n_maps < 1 || n_envs < 1 || !opts || !out) return fail(LLE_INVALID_ARGUMENT, "bad argument");
     if (opts->reward_dim != 1 && opts->reward_dim != 4) return fail(LLE_INVALID_ARGUMENT, "reward_dim must be 1 or 4");
+    if (opts->obs_dtype != LLE_DTYPE_F32 && opts->obs_dtype != LLE_DTYPE_I8) return fail(LLE_INVALID_ARGUMENT, "obs_dtype must be LLE_DTYPE_F32 or LLE_DTYPE_I8");
+    if (opts->obs_dtype == LLE_DTYPE_I8 && (opts->obs_type == LLE_OBS_PARTIAL || opts->obs_type == LLE_OBS_STATE))
+        return fail(LLE_INVALID_ARGUMENT, "obs_dtype int8: only layered and perspective observations (partial and state are float32)");
     auto v = std::unique_ptr<lle_vec, int (*)(lle_vec*)>(new lle_vec(), lle_vec_destroy);
     v->opts = *opts;
     v->device = opts->device;
-    // The caller's maps are compiled for the plain layered observation; other observation types get their own device
-    // tables (channel layout, static planes, patch and agent-plane tables) from the same map text.
-    const ObsSpec spec{opts->obs_type, opts->obs_param};
+    // The caller's maps are compiled for the plain layered f32 observation; other observation types and int8 observations get
+    // their own device tables (channel layout, static planes, patch and agent-plane tables) from the same map text.
+    const ObsSpec spec{opts->obs_type, opts->obs_param, opts->obs_dtype};
+    v->i8 = opts->obs_dtype == LLE_DTYPE_I8;
+    const int64_t es = v->i8 ? 1 : 4;  // bytes per observation element
     std::vector<const CompiledMap*> cms;
     if (spec == ObsSpec()) {
         for (int k = 0; k < n_maps; ++k) cms.push_back(&maps[k]->cm);
@@ -647,7 +677,9 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         if (opts->pbrs && opts->reward_dim == 4) v->R = 5;  // np.concat((reward, [potential_reward])) (reward_strategy.py:153)
     }
     v->L = lle_state_layout(v->A, v->G, v->NBmax, v->max_beam_len, v->JE > 0, opts->pbrs != 0);
-    v->obs_stride = spec.kind == LLE_OBS_STATE ? (int64_t)v->S : ((int64_t)m0.header().obs_floats + 3) / 4 * 4;
+    // rows are padded to 16 bytes: every row and tile is a legal cp.async.bulk source and destination
+    const int64_t per16 = 16 / es;
+    v->obs_stride = spec.kind == LLE_OBS_STATE ? (int64_t)v->S : ((int64_t)m0.header().obs_floats + per16 - 1) / per16 * per16;
     v->render = opts->write_obs && spec.kind != LLE_OBS_STATE;  // whether the tile renderer runs
 
     LLE_CUDA(cudaSetDevice(v->device));
@@ -655,12 +687,15 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
     LLE_CUDA(cudaGetDeviceProperties(&prop, v->device));
 
     // ---- work decomposition and observation tiling.  One bulk store should move a few KB; a warp takes a
-    // ticket for `group` consecutive worlds, computes them, then streams their observation tiles.
+    // ticket for `group` consecutive worlds, computes them, then streams their observation tiles.  Sizes are reasoned about in
+    // bytes (`es` per element): an int8 row takes a quarter of the bytes of the f32 row and is tiled like an f32 row of that size.
     v->Wd = 1;
     while (v->Wd < v->A) v->Wd *= 2;
     // at least 2 lanes per world (16 worlds per pass, 16 per ticket).  Measured on B200 with narrow-grid pipelining
     // (us/step, lanes per world 1 / 2 / 4): level 1: 40.7 / 40.3 / 45.4; level 3: 51.8 / 51.5 / 58.0
-    const bool small_obs = v->obs_stride * 4 < 2048;  // tiny observations: the logic dominates, pack more worlds per pass
+    // tiny observations: the logic dominates, pack more worlds per pass.  In bytes: a level-6 int8 row (1,872 B) is small and
+    // runs on the thread-per-world kernel (level 6 x 65,536 on one B200: 45.5 us per step there, 65.9 on the fast kernel)
+    const bool small_obs = v->obs_stride * es < 2048;
     v->Wd = std::max(v->Wd, std::min(32, env_int("LLE_B200_MIN_WD", small_obs ? 1 : 2)));
     const int64_t stride = v->obs_stride;
     // 4-8 KB per bulk store; partial observations: up to 9.6 KB, one tile buffer and 16 worlds per ticket, which keeps five
@@ -677,9 +712,10 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
     // one: 3x3 52.5 / 58-67, 5x5 90 / 85, 7x7 166 / 98 - with 2,048 tickets a launch is one wave of warps and the step takes as
     // long as one ticket, so larger windows (more rounds per ticket) stay on the general kernel, which has four times the warps.
     const bool tiny_partial = partial_obs && tiny_record && (stride * 4 < 2048 || env_int("LLE_B200_TINY_PARTIAL", 0));
-    const int64_t kTileTargetFloats = env_int("LLE_B200_TILE_TARGET", partial_obs ? 2400 : small_obs ? 2048 : 1024);
+    // (targets and limits in 4-byte units, as measured on f32; elements of the vec's type below)
+    const int64_t kTileTargetFloats = env_int("LLE_B200_TILE_TARGET", partial_obs ? 2400 : small_obs ? 2048 : 1024) * 4 / es;
     // the partial renderer builds whole worlds (all agents' windows) in one tile: allow up to 48 KB per warp
-    const int64_t kTileMaxFloats = spec.kind == LLE_OBS_PARTIAL ? 12288 : 6144;
+    const int64_t kTileMaxFloats = (spec.kind == LLE_OBS_PARTIAL ? 12288 : 6144) * 4 / es;
     if (spec.kind == LLE_OBS_PARTIAL && stride > kTileMaxFloats)
         return fail(LLE_LIMIT_EXCEEDED, "partial observation of one world exceeds 48 KB (n_agents * (2 n_agents + 3) * size^2 floats)");
     if (stride <= kTileMaxFloats) {
@@ -691,7 +727,7 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         v->n_buf = 1;
     } else {
         v->E = 1;
-        v->chunk_floats = lle_chunk_floats(stride);  // <= 12 KB, balanced (static_map.h)
+        v->chunk_floats = lle_chunk_elems(stride, (int)es);  // <= 12 KB, balanced (static_map.h)
         v->n_chunks = (int)((stride + v->chunk_floats - 1) / v->chunk_floats);
         v->tile_floats = v->chunk_floats;
         // A ticket walks its worlds chunk by chunk, so the two tile buffers are rebuilt from the static plane twice per
@@ -701,7 +737,7 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         // Tickets are also the grain of the dataflow ordering between overlapped steps, so very large ones stall the
         // pipeline (64x64 x 131,072: 2.02e7 / 2.07e7 / 1.72e7 env-steps/s with 8 / 16 / 32): at most 6 MB per ticket.
         v->group = 32;
-        while (v->group > std::max(8, 32 / v->Wd) && (v->N_pad / v->group < 2048 || (int64_t)v->group * stride * 4 > (6 << 20))) v->group >>= 1;
+        while (v->group > std::max(8, 32 / v->Wd) && (v->N_pad / v->group < 2048 || (int64_t)v->group * stride * es > (6 << 20))) v->group >>= 1;
         v->n_buf = 2;
     }
     {
@@ -709,7 +745,7 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         if (g >= v->E && g >= 32 / v->Wd && g <= 32 && (g & (g - 1)) == 0) v->group = g;
     }
     auto warp_smem_for = [&](int n_buf) {
-        size_t bytes = (size_t)n_buf * v->tile_floats * 4;             // tiles
+        size_t bytes = (size_t)n_buf * v->tile_floats * es;            // tiles
         bytes += (size_t)v->group * v->L.stride * 4;                   // records of the group
         bytes += (size_t)n_buf * v->E * v->L.stride * 4;               // records applied to the tiles
         bytes += (size_t)(2 * n_buf * v->E + n_buf + v->group) * 4;    // tags + map ids + fresh flags
@@ -734,7 +770,17 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         for (const auto& m : v->variant_maps) v->by_feature = v->by_feature && (int)m.header().n_patch <= v->feature_limit;
     }
     int blocks_per_sm = -1;  // the grid is shared by the three modes: size it for the most demanding one
-    if (v->fast) {
+    if (v->i8 && v->fast) {
+        LLE_CUDA((configure_kernel<MODE_STEP, 1, false, int8_t>(v->smem, &blocks_per_sm)));
+        LLE_CUDA((configure_kernel<MODE_STEP, 1, true, int8_t>(v->smem, &blocks_per_sm)));
+        LLE_CUDA((configure_kernel<MODE_RESET, 1, false, int8_t>(v->smem, &blocks_per_sm)));
+        LLE_CUDA((configure_kernel<MODE_SET_STATE, 1, false, int8_t>(v->smem, &blocks_per_sm)));
+    } else if (v->i8) {
+        LLE_CUDA((configure_kernel<MODE_STEP, 0, false, int8_t>(v->smem, &blocks_per_sm)));
+        LLE_CUDA((configure_kernel<MODE_STEP, 0, true, int8_t>(v->smem, &blocks_per_sm)));
+        LLE_CUDA((configure_kernel<MODE_RESET, 0, false, int8_t>(v->smem, &blocks_per_sm)));
+        LLE_CUDA((configure_kernel<MODE_SET_STATE, 0, false, int8_t>(v->smem, &blocks_per_sm)));
+    } else if (v->fast) {
         LLE_CUDA((configure_kernel<MODE_STEP, 1>(v->smem, &blocks_per_sm)));
         LLE_CUDA((configure_kernel<MODE_STEP, 1, true>(v->smem, &blocks_per_sm)));
         LLE_CUDA((configure_kernel<MODE_RESET, 1>(v->smem, &blocks_per_sm)));
@@ -757,6 +803,10 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
     if (v->tiny) {
         // worlds per tile / bulk store (measured on 2^20 5x5 worlds, us per step: 4: 232, 8: 243, 16: 343, 32: 558 - occupancy)
         int e_default = 4;
+        // int8 rows: more worlds per tile, up to 4 KB and 16 worlds (measured on 2^20 5x5 worlds, 208 B rows, us per step: 4: 157.7,
+        // 8: 145.4, 16: 135.7, 32: 142.8; level 1 x 65,536, 944 B rows: 4: 14.7, 16: 14.4)
+        if (v->i8)
+            while (e_default < 16 && 2 * e_default * stride <= 4096) e_default *= 2;
         if (tiny_partial) {  // the largest tile of at most 13 KB (level 6 3x3: 8 worlds; measured 2 / 4 / 8: 60.8 / 57.0 / 52.5 us)
             e_default = 1;
             while (e_default < 32 && 2 * e_default * stride * 4 <= 13312) e_default *= 2;
@@ -764,7 +814,7 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         int e = env_int("LLE_B200_TINY_E", e_default);
         v->tiny_E = (e >= (tiny_partial ? 1 : 4) && e <= 32 && (e & (e - 1)) == 0) ? e : e_default;
         auto tiny_bytes = [&]() {  // the records' columns + the prefetched next records, list pointers, list lengths, the tile
-            const size_t bytes = 2 * (size_t)v->L.stride * 32 * 4 + 32 * 8 + 32 * 4 + (tiny_partial ? 32 * 8 : 0) + (size_t)v->tiny_E * stride * 4;
+            const size_t bytes = 2 * (size_t)v->L.stride * 32 * 4 + 32 * 8 + 32 * 4 + (tiny_partial ? 32 * 8 : 0) + (size_t)v->tiny_E * stride * es;
             return (bytes + 127) / 128 * 128;
         };
         v->tiny_chunk = std::max(1, std::min(64, env_int("LLE_B200_TINY_CHUNK", 1)));
@@ -779,7 +829,14 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
             if (e2 != cudaSuccess) return e2;
             return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tb, kern, kThreads, v->tiny_smem);
         };
-        switch (v->A * 2 + (tiny_partial ? 1 : 0)) {
+        if (v->i8) {
+            switch (v->A) {
+                case 1: LLE_CUDA(configure(lle_tiny_step_kernel<1, false, int8_t>)); break;
+                case 2: LLE_CUDA(configure(lle_tiny_step_kernel<2, false, int8_t>)); break;
+                case 3: LLE_CUDA(configure(lle_tiny_step_kernel<3, false, int8_t>)); break;
+                default: LLE_CUDA(configure(lle_tiny_step_kernel<4, false, int8_t>)); break;
+            }
+        } else switch (v->A * 2 + (tiny_partial ? 1 : 0)) {
             case 2: LLE_CUDA(configure(lle_tiny_step_kernel<1, false>)); break;
             case 3: LLE_CUDA(configure(lle_tiny_step_kernel<1, true>)); break;
             case 4: LLE_CUDA(configure(lle_tiny_step_kernel<2, false>)); break;
@@ -852,7 +909,8 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
     }
     const size_t Np = (size_t)v->N_pad;
     LLE_CUDA(dalloc(&v->d_records, (size_t)v->L.stride * Np));
-    if (opts->write_obs) LLE_CUDA(dalloc(&v->d_obs, (size_t)v->obs_stride * Np));
+    if (opts->write_obs && v->i8) LLE_CUDA(dalloc(&v->d_obs_i8, (size_t)v->obs_stride * Np));
+    else if (opts->write_obs) LLE_CUDA(dalloc(&v->d_obs, (size_t)v->obs_stride * Np));
     v->hdr0 = m0.header();
     LLE_CUDA(dalloc(&v->d_state, (size_t)v->S * Np));
     LLE_CUDA(dalloc(&v->d_avail, (size_t)v->A * 5 * Np));
@@ -891,6 +949,7 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         so.state_type = LLE_OBS_STATE; so.state_param = 0;
         so.write_obs = 1;
         so.episode_stats = 0;
+        so.obs_dtype = LLE_DTYPE_F32;  // the state observation stays float32
         lle_vec* sh = nullptr;
         if (int rc2 = lle_vec_create(maps, n_maps, map_of_env, n_envs, &so, &sh)) return rc2;
         if (sh->L.stride != v->L.stride || sh->N_pad != v->N_pad || (sh->d_map_of_env == nullptr) != (v->d_map_of_env == nullptr)) {
@@ -930,6 +989,8 @@ int lle_vec_get_buffers(lle_vec* v, lle_vec_buffers* out) {
     out->map_index = v->d_map_of_env;
     out->n_variants = v->n_variants;
     out->info = v->d_info; out->ep_return = v->d_ep_return; out->ep_length = v->d_ep_length; out->last_return = v->d_last_return; out->last_length = v->d_last_length;
+    out->obs_i8 = v->d_obs_i8;
+    out->obs_dtype = v->opts.obs_dtype;
     if (v->shadow) {
         const lle_vec* sh = v->shadow;
         out->state_obs = sh->d_obs; out->state_obs_stride = sh->obs_stride;
@@ -957,7 +1018,7 @@ int swap_map(lle_vec* v, int map_index, const std::vector<SourceState>& sources,
              CompiledMap* out_cm) {
     CompiledMap cm;
     try {
-        cm = compile_map(v->map_texts[(size_t)map_index], ObsSpec{v->opts.obs_type, v->opts.obs_param}, &sources, exits);
+        cm = compile_map(v->map_texts[(size_t)map_index], ObsSpec{v->opts.obs_type, v->opts.obs_param, v->opts.obs_dtype}, &sources, exits);
     } catch (const MapError& e) {
         return fail(e.status, e.what());
     }
@@ -1167,7 +1228,10 @@ int lle_vec_fetch(lle_vec* v, int which, size_t offset, size_t bytes, void* host
     const void* src = nullptr;
     size_t size = 0;
     switch (which) {
-        case LLE_BUF_OBS: src = v->d_obs; size = N * (size_t)v->obs_stride * 4; break;
+        case LLE_BUF_OBS:
+            src = v->i8 ? (const void*)v->d_obs_i8 : (const void*)v->d_obs;
+            size = N * (size_t)v->obs_stride * (v->i8 ? 1 : 4);
+            break;
         case LLE_BUF_STATE: src = v->d_state; size = N * (size_t)v->S * 4; break;
         case LLE_BUF_AVAIL: src = v->d_avail; size = N * A * 5; break;
         case LLE_BUF_REWARD: src = v->d_reward; size = N * (size_t)v->R * 4; break;

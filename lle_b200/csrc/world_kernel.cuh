@@ -45,7 +45,7 @@ struct MapDev {
     const LleCellBeams* cellbeams;
     const LleBeam* beams;
     const LlePatch* patches;
-    const float* stat;
+    const float* stat;  // the static plane; int8_t elements when the map was compiled for an int8 observation
     const LleAgentPlane* agent_planes;
     const uint32_t* chunk_tbl;
     int n_patch, NB, obs_floats, n_ap;
@@ -157,7 +157,16 @@ struct KParams {
     int32_t* ep_length;    // [N_pad]     its steps so far
     float* last_return;    // [N_pad][R]  the same two of the last finished episode
     int32_t* last_length;  // [N_pad]
+    int8_t* obs_i8;        // the observation rows of an int8 vec (lle_vec_options.obs_dtype; obs is then null).  Elements of
+                           // either type are counted alike: obs_stride, tile_floats and chunk_floats count int8 elements there
 };
+
+// The observation rows as the kernel's element type OT (float, or int8_t for an int8 vec)
+template <typename OT>
+__device__ __forceinline__ OT* obs_rows(const KParams& p) {
+    if constexpr (sizeof(OT) == 1) return p.obs_i8;
+    else return p.obs;
+}
 
 // ---- PTX wrappers (TMA 1-D bulk store through the async proxy) ----------------------------------------
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
@@ -614,25 +623,26 @@ __device__ __forceinline__ uint32_t rec_pos(const uint32_t* rec, int a) {
 }
 
 // Per-lane register copy of the first 64 patch entries of the map being rendered (entries lane and lane + 32):
-// the float index, the static value to restore, and where in a record the controlling bit lives.
+// the element index, the static value to restore (as the tile's element type OT), and where in a record the controlling bit lives.
+template <typename OT>
 struct PatchCache {
     uint32_t idx0, idx1;
-    float stat0, stat1;
+    OT stat0, stat1;
     uint16_t word0, word1;  // record word holding the bit
     uint8_t bit0, bit1, gem0, gem1;
     bool valid0, valid1;
     __device__ __forceinline__ void load(const MapDev& rm, const LleStateLayout& L, int lane) {
         valid0 = lane < rm.n_patch;
         valid1 = lane + 32 < rm.n_patch;
-        idx0 = idx1 = 0; stat0 = stat1 = 0.f; word0 = word1 = 0; bit0 = bit1 = gem0 = gem1 = 0;
+        idx0 = idx1 = 0; stat0 = stat1 = (OT)0; word0 = word1 = 0; bit0 = bit1 = gem0 = gem1 = 0;
         if (valid0) {
             const LlePatch pe = rm.patches[lane];
-            idx0 = pe.idx; stat0 = (float)pe.stat; gem0 = pe.src == 0xFF; bit0 = pe.bit & 31;
+            idx0 = pe.idx; stat0 = (OT)pe.stat; gem0 = pe.src == 0xFF; bit0 = pe.bit & 31;
             word0 = (uint16_t)(gem0 ? L.w_gems + (pe.bit >> 5) : L.w_on + pe.src * L.on_words + (pe.bit >> 5));
         }
         if (valid1) {
             const LlePatch pe = rm.patches[lane + 32];
-            idx1 = pe.idx; stat1 = (float)pe.stat; gem1 = pe.src == 0xFF; bit1 = pe.bit & 31;
+            idx1 = pe.idx; stat1 = (OT)pe.stat; gem1 = pe.src == 0xFF; bit1 = pe.bit & 31;
             word1 = (uint16_t)(gem1 ? L.w_gems + (pe.bit >> 5) : L.w_on + pe.src * L.on_words + (pe.bit >> 5));
         }
     }
@@ -641,21 +651,28 @@ struct PatchCache {
     __device__ __forceinline__ bool lit1(const uint32_t* rec) const { return (((rec[word1] >> bit1) & 1u) ^ gem1) != 0; }
 };
 
-// (Re)build floats [lo, hi) of one world's block from the map's static plane (observations.py:216-237) with
-// asynchronous copies; pad floats beyond C*H*W are zero.  Completion: cp_async_wait_all() + __syncwarp().
-__device__ __forceinline__ void tile_rebuild_async(float* sub_tile, const MapDev& rm, int lo, int hi, int lane) {
+// (Re)build elements [lo, hi) of one world's block from the map's static plane (observations.py:216-237) with
+// asynchronous copies; pad elements beyond C*H*W are zero.  Completion: cp_async_wait_all() + __syncwarp().
+// int8: the plane is zero-padded to the row stride and lo, hi are multiples of 16, so every piece is one 16-byte copy.
+template <typename OT>
+__device__ __forceinline__ void tile_rebuild_async(OT* sub_tile, const MapDev& rm, int lo, int hi, int lane) {
     const int nf = hi - lo;
-    for (int f = lane * 4; f < nf; f += 128) {
-        const int gi = lo + f;
-        if (gi + 3 < rm.obs_floats) {
-            cp_async16(sub_tile + f, rm.stat + gi);
-        } else {
-            float4 v;
-            v.x = gi + 0 < rm.obs_floats ? __ldg(rm.stat + gi + 0) : 0.f;
-            v.y = gi + 1 < rm.obs_floats ? __ldg(rm.stat + gi + 1) : 0.f;
-            v.z = gi + 2 < rm.obs_floats ? __ldg(rm.stat + gi + 2) : 0.f;
-            v.w = gi + 3 < rm.obs_floats ? __ldg(rm.stat + gi + 3) : 0.f;
-            *reinterpret_cast<float4*>(sub_tile + f) = v;
+    if constexpr (sizeof(OT) == 1) {
+        const int8_t* stat = reinterpret_cast<const int8_t*>(rm.stat);
+        for (int f = lane * 16; f < nf; f += 512) cp_async16(sub_tile + f, stat + lo + f);
+    } else {
+        for (int f = lane * 4; f < nf; f += 128) {
+            const int gi = lo + f;
+            if (gi + 3 < rm.obs_floats) {
+                cp_async16(sub_tile + f, rm.stat + gi);
+            } else {
+                float4 v;
+                v.x = gi + 0 < rm.obs_floats ? __ldg(rm.stat + gi + 0) : 0.f;
+                v.y = gi + 1 < rm.obs_floats ? __ldg(rm.stat + gi + 1) : 0.f;
+                v.z = gi + 2 < rm.obs_floats ? __ldg(rm.stat + gi + 2) : 0.f;
+                v.w = gi + 3 < rm.obs_floats ? __ldg(rm.stat + gi + 3) : 0.f;
+                *reinterpret_cast<float4*>(sub_tile + f) = v;
+            }
         }
     }
 }
@@ -807,7 +824,10 @@ __device__ __forceinline__ void launch_epilogue(const KParams& p, bool is_step) 
 // KIND: 0 general, 1 FAST (above), 2 general with the feature-driven renderer of partial observations (sparse maps).
 // PARTS: the step kernel of a parts loop (lle_vec_parts_*): tickets wait for their part's actions and completed parts are
 // published to the host.  A separate instantiation: the plain step kernel carries none of it.
-template <int MODE, int KIND, bool PARTS = false>
+// OT: the observation's element type, float or int8_t (lle_vec_options.obs_dtype).  An int8 vec renders the same tiles in bytes:
+// the static plane, patch values and one-hots are byte stores and every bulk store moves a quarter of the bytes.  Partial
+// observations are float only.
+template <int MODE, int KIND, bool PARTS = false, typename OT = float>
 __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const KParams p) {
     constexpr bool FAST = KIND == 1;
     constexpr bool BY_FEATURE = KIND == 2;
@@ -816,7 +836,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
     const LleStateLayout L = p.L;
     const int A = p.A, stride = L.stride;
     uint8_t* wbase = smem_raw + (size_t)warp * p.warp_smem_bytes;
-    float* tiles = reinterpret_cast<float*>(wbase);                                          // [n_buf][tile_floats]
+    OT* tiles = reinterpret_cast<OT*>(wbase);                                                // [n_buf][tile_floats]
     uint32_t* recs = reinterpret_cast<uint32_t*>(tiles + (size_t)p.n_buf * p.tile_floats);   // [group][stride]
     uint32_t* applied = recs + (size_t)p.group * stride;                                     // [n_buf][E][stride]
     int32_t* tags = reinterpret_cast<int32_t*>(applied + (size_t)p.n_buf * p.E * stride);    // [n_buf][E] map id, [n_buf] chunk
@@ -839,7 +859,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
     const int sub = lane / Wd, gl = w.gl;
     int bound_map = -1;       // map bound to this lane's World
     MapDev rm;                // map bound for rendering (warp-uniform)
-    PatchCache pc;
+    PatchCache<OT> pc;
     int render_map = -1;
     int buf = 0;
     bool tile_fresh = true;  // FAST: the tile was just (pre)built from the static plane
@@ -1220,26 +1240,26 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                         }
                         const uint32_t* cur = recs + (size_t)g * stride;
                         const uint32_t* old = applied + (size_t)s * stride;
-                        float* sub = tiles + (size_t)s * p.obs_stride;
+                        OT* sub = tiles + (size_t)s * p.obs_stride;
                         if (!((fresh_bits >> s) & 1u)) {  // un-patch what the previous occupant had lit and this one has not
                             for (int k = e; k < rm.n_patch; k += Pr) {
                                 const LlePatch pe = rm.patches[k];
-                                if (rec_lit(old, L, pe) && !rec_lit(cur, L, pe)) sub[pe.idx] = (float)pe.stat;
+                                if (rec_lit(old, L, pe) && !rec_lit(cur, L, pe)) sub[pe.idx] = (OT)pe.stat;
                             }
                             for (int a = e; a < A; a += Pr) {
                                 const uint32_t op = rec_pos(old, a);
-                                sub[a * p.HW + (int)(op >> 8) * p.W + (int)(op & 0xFFu)] = 0.0f;
+                                sub[a * p.HW + (int)(op >> 8) * p.W + (int)(op & 0xFFu)] = (OT)0;
                             }
                         }
                         fresh_bits &= ~(p.E >= 32 ? ~0u : ((1u << p.E) - 1u));
                         __syncwarp();
                         for (int k = e; k < rm.n_patch; k += Pr) {  // every lit entry is rewritten (aliasing entries, see below)
                             const LlePatch pe = rm.patches[k];
-                            if (rec_lit(cur, L, pe)) sub[pe.idx] = 1.0f;
+                            if (rec_lit(cur, L, pe)) sub[pe.idx] = (OT)1;
                         }
                         for (int a = e; a < A; a += Pr) {
                             const uint32_t np = rec_pos(cur, a);
-                            sub[a * p.HW + (int)(np >> 8) * p.W + (int)(np & 0xFFu)] = 1.0f;
+                            sub[a * p.HW + (int)(np >> 8) * p.W + (int)(np & 0xFFu)] = (OT)1;
                         }
                         // the tile now shows worlds [tix*E, tix*E + E) of the group: their records are contiguous
                         for (int k = lane; k < p.E * stride; k += 32) applied[k] = recs[(size_t)tix * p.E * stride + k];
@@ -1248,7 +1268,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                 for (int s = 0; s < (parallel ? 0 : p.E); ++s) {
                     const int g = tix * p.E + s;
                     const uint32_t* cur = recs + (size_t)g * stride;
-                    float* sub = tiles + (size_t)s * p.obs_stride;
+                    OT* sub = tiles + (size_t)s * p.obs_stride;
                     uint32_t* old = applied + (size_t)s * stride;
                     int mid = 0;
                     if (multi) {
@@ -1269,7 +1289,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                         // un-patch what the previous occupant had lit and this one has not
                         if (lane < A) {
                             const uint32_t op = rec_pos(old, lane);
-                            sub[agent_base + (int)(op >> 8) * p.W + (int)(op & 0xFFu)] = 0.0f;  // agent planes have no static content
+                            sub[agent_base + (int)(op >> 8) * p.W + (int)(op & 0xFFu)] = (OT)0;  // agent planes have no static content
                         }
                         if (pc.valid0 && !now0 && pc.lit0(old)) sub[pc.idx0] = pc.stat0;
                         if (pc.valid1 && !now1 && pc.lit1(old)) sub[pc.idx1] = pc.stat1;
@@ -1278,11 +1298,11 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                     __syncwarp();
                     // patch.  Every lit entry is rewritten so that entries aliasing one cell (crossing beams of one colour,
                     // colours >= n_agents) stay correct whatever was un-patched above; then the agents (observations.py:264-265).
-                    if (now0) sub[pc.idx0] = 1.0f;
-                    if (now1) sub[pc.idx1] = 1.0f;
+                    if (now0) sub[pc.idx0] = (OT)1;
+                    if (now1) sub[pc.idx1] = (OT)1;
                     if (lane < A) {
                         const uint32_t np = rec_pos(cur, lane);
-                        sub[agent_base + (int)(np >> 8) * p.W + (int)(np & 0xFFu)] = 1.0f;
+                        sub[agent_base + (int)(np >> 8) * p.W + (int)(np & 0xFFu)] = (OT)1;
                     }
                     if (lane < stride) old[lane] = cur[lane];
                 }
@@ -1291,8 +1311,8 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                 if (lane == 0) {
                     // evict-first: the rows stream through L2 to HBM (491 MB per level-6 step of 65,536 worlds, four times the L2)
                     // and should not push out the records, flags and small outputs the next step reads and rewrites
-                    bulk_store_hint(p.obs + (env0 + (int64_t)tix * p.E) * p.obs_stride, tiles, (uint32_t)(p.E * p.obs_stride) * 4u,
-                                    l2_evict_first_policy());
+                    bulk_store_hint(obs_rows<OT>(p) + (env0 + (int64_t)tix * p.E) * p.obs_stride, tiles,
+                                    (uint32_t)(p.E * p.obs_stride) * (uint32_t)sizeof(OT), l2_evict_first_policy());
                     bulk_commit();
                     if (p.timeline) {
                         t_last = globaltimer_ns();
@@ -1307,7 +1327,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
             owed = true; owed_ticket = ticket; owed_seq = my_seq;
             continue;
         } else {
-        if (p.obs_kind == LLE_OBS_PARTIAL) {
+        if constexpr (sizeof(OT) == 4) if (p.obs_kind == LLE_OBS_PARTIAL) {
             // PartialGenerator.observe (observations.py:331-350): per agent a (2A+3, size, size) window centred on it; channels
             // agents, WALL, lasers, GEM, EXIT.  One lane per (agent, window cell): it looks the map cell up once and
             // writes the few non-zero channels into a zero-filled tile, which leaves with one bulk store per E worlds.
@@ -1315,7 +1335,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
             const float inv_s2 = 1.0f / (float)s2, inv_sz = 1.0f / (float)sz;
             const int n_tiles = p.group / p.E, tile_len = p.E * (int)p.obs_stride;
             for (int tix = 0; tix < n_tiles; ++tix) {
-                float* tile = tiles + (size_t)buf * p.tile_floats;
+                OT* tile = tiles + (size_t)buf * p.tile_floats;
                 if (lane == 0) {
                     if (p.n_buf == 2) bulk_wait_read<1>();
                     else bulk_wait_read<0>();
@@ -1331,7 +1351,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                         render_map = mid;
                     }
                     const uint32_t* cur = recs + (size_t)g * stride;
-                    float* sub = tile + (size_t)s * p.obs_stride;
+                    OT* sub = tile + (size_t)s * p.obs_stride;
                     if constexpr (BY_FEATURE) {
                         // Sparse maps (the host selects this kernel when every map has at most 2 s^2 features): one lane per
                         // (agent, feature) — the map's walls, exits, sources, gems and laser tiles — instead of one per
@@ -1360,7 +1380,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                         const int c = i * p.W + j;
                         const uint32_t info = rm.cellinfo[c];
                         if (!(info & (7u | (1u << 24)))) continue;  // plain floor, no beam: nothing but agents (below)
-                        float* o = sub + a * Cp * s2 + r;
+                        OT* o = sub + a * Cp * s2 + r;
                         const uint32_t kind = info & 7u;
                         if (kind == LLE_T_WALL) {
                             // WALL = n_agents; wall_pos holds the walls and the v1 sources (parser_v1.rs:22-25), but not
@@ -1420,7 +1440,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
             const int lo = chunk * p.chunk_floats;  // float range [lo, hi) of one world's block
             const int hi = min(lo + p.chunk_floats, (int)p.obs_stride);
             for (int tix = 0; tix < tiles_per_group; ++tix) {
-                float* tile = tiles + (size_t)buf * p.tile_floats;
+                OT* tile = tiles + (size_t)buf * p.tile_floats;
                 // the bulk store that last read this buffer must have finished reading it
                 if (lane == 0) {
                     if (p.n_buf == 2) bulk_wait_read<1>();
@@ -1436,7 +1456,7 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                         render_map = mid;
                         pc.load(rm, L, lane);
                     }
-                    float* sub_tile = tile + (size_t)s * p.obs_stride;
+                    OT* sub_tile = tile + (size_t)s * p.obs_stride;
                     uint32_t* old = applied + ((size_t)buf * p.E + s) * stride;
                     const uint32_t* cur = recs + (size_t)g * stride;
                     const int slot_id = buf * p.E + s;
@@ -1461,29 +1481,29 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                             const LleAgentPlane ap = rm.agent_planes[k];
                             const uint32_t op = rec_pos(old, (int)ap.agent);
                             const int idx = (int)ap.base + (int)(op >> 8) * p.W + (int)(op & 0xFFu);
-                            if (whole || (idx >= lo && idx < hi)) sub_tile[idx - lo] = 0.0f;  // agent planes have no static content
+                            if (whole || (idx >= lo && idx < hi)) sub_tile[idx - lo] = (OT)0;  // agent planes have no static content
                         }
                         if (v0 && in0 && pc.lit0(old) && !now0) sub_tile[pc.idx0 - lo] = pc.stat0;
                         if (v1 && in1 && pc.lit1(old) && !now1) sub_tile[pc.idx1 - lo] = pc.stat1;
                         for (int k = k_begin + lane; k < k_end; k += 32) {
                             const LlePatch pe = rm.patches[k];
-                            if (rec_lit(old, L, pe) && !rec_lit(cur, L, pe)) sub_tile[pe.idx - lo] = (float)pe.stat;
+                            if (rec_lit(old, L, pe) && !rec_lit(cur, L, pe)) sub_tile[pe.idx - lo] = (OT)pe.stat;
                         }
                     }
                     __syncwarp();
                     // patch.  Every lit entry is rewritten so that entries aliasing one cell (crossing beams of one colour,
                     // colours >= n_agents) stay correct whatever was un-patched above; then the agents (observations.py:264-265).
-                    if (now0 && in0) sub_tile[pc.idx0 - lo] = 1.0f;
-                    if (now1 && in1) sub_tile[pc.idx1 - lo] = 1.0f;
+                    if (now0 && in0) sub_tile[pc.idx0 - lo] = (OT)1;
+                    if (now1 && in1) sub_tile[pc.idx1 - lo] = (OT)1;
                     for (int k = k_begin + lane; k < k_end; k += 32) {
                         const LlePatch pe = rm.patches[k];
-                        if (rec_lit(cur, L, pe)) sub_tile[pe.idx - lo] = 1.0f;
+                        if (rec_lit(cur, L, pe)) sub_tile[pe.idx - lo] = (OT)1;
                     }
                     for (int k = lane; k < rm.n_ap; k += 32) {
                         const LleAgentPlane ap = rm.agent_planes[k];
                         const uint32_t np = rec_pos(cur, (int)ap.agent);
                         const int idx = (int)ap.base + (int)(np >> 8) * p.W + (int)(np & 0xFFu);
-                        if (whole || (idx >= lo && idx < hi)) sub_tile[idx - lo] = 1.0f;
+                        if (whole || (idx >= lo && idx < hi)) sub_tile[idx - lo] = (OT)1;
                     }
                     for (int k = lane; k < stride; k += 32) old[k] = cur[k];
                     if (lane == 0) { tags[slot_id] = mid; fresh[slot_id] = 0; }
@@ -1493,8 +1513,8 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
                 __syncwarp();
                 if (lane == 0) {
                     const int64_t first_env = env0 + (whole ? tix * p.E : tix);
-                    float* dst = p.obs + first_env * p.obs_stride + lo;
-                    const uint32_t bytes = (uint32_t)((whole ? p.E * (int)p.obs_stride : (hi - lo)) * 4);
+                    OT* dst = obs_rows<OT>(p) + first_env * p.obs_stride + lo;
+                    const uint32_t bytes = (uint32_t)((whole ? p.E * (int)p.obs_stride : (hi - lo)) * (int)sizeof(OT));
                     bulk_store(dst, tile, bytes);
                     bulk_commit();
                     if (p.timeline) {

@@ -11,7 +11,7 @@ from typing import Sequence
 import torch
 
 from .types import obs_spec
-from .vec_world import Map, VecWorld
+from .vec_world import Map, VecWorld, _obs_dtype
 
 
 class VecLLE:
@@ -24,12 +24,12 @@ class VecLLE:
     def __init__(self, maps, n_envs: int, *, map_of_env: Sequence[int] | None = None, device=0, multi_objective: bool = False,
                  walkable_lasers: bool = True, auto_reset: bool = True, seed: int = 0, env_id_base: int = 0, write_obs: bool = True,
                  extras=None, pbrs: dict | None = None, obs_type: str = "layered", padding_size: int = 0,
-                 randomize_lasers: bool = False, state_type: str = "state", episode_stats: bool = False):
+                 randomize_lasers: bool = False, state_type: str = "state", episode_stats: bool = False, obs_dtype=torch.float32):
         self.world = VecWorld(maps, n_envs, map_of_env=map_of_env, device=device, reward_dim=4 if multi_objective else 1,
                               walkable_lasers=walkable_lasers, auto_reset=auto_reset, lle_semantics=True, write_obs=write_obs,
                               seed=seed, env_id_base=env_id_base, extras=extras, pbrs=pbrs, obs_type=obs_type,
                               padding_size=padding_size, randomize_lasers=randomize_lasers, state_type=state_type,
-                              episode_stats=episode_stats)
+                              episode_stats=episode_stats, obs_dtype=obs_dtype)
         if self.world.obs_invalid and write_obs:
             raise IndexError("index out of bounds: a laser colour selects a channel past the last layer")
         w = self.world
@@ -214,6 +214,12 @@ class Builder:
         """Builder.obs_type (builder.py:42-49): any ObservationType value but "rgb-image"."""
         obs_spec(obs_type, padding_size)  # ValueError / NotImplementedError
         self._kw["obs_type"], self._kw["padding_size"] = obs_type, int(padding_size)
+        return self
+
+    def obs_dtype(self, dtype=torch.float32):
+        """Element type of the observation: torch.float32 (default) or torch.int8 (also "float32" / "int8"), a quarter of the
+        bytes for layered and perspective observations (VecWorld's obs_dtype)."""
+        self._kw["obs_dtype"] = _obs_dtype(dtype)  # ValueError
         return self
 
     def episode_stats(self, enabled: bool = True):

@@ -89,6 +89,15 @@ class Map:
                  buf[7 * k + 6]) for k in range(n.value)]
 
 
+def _obs_dtype(dtype) -> torch.dtype:
+    """torch.float32 / torch.int8, or their names."""
+    named = {"float32": torch.float32, "int8": torch.int8}
+    dt = named.get(dtype, dtype) if isinstance(dtype, str) else dtype
+    if dt not in (torch.float32, torch.int8):
+        raise ValueError(f"obs_dtype must be torch.float32 or torch.int8 (or 'float32' / 'int8'), got {dtype!r}")
+    return dt
+
+
 class _DevArray:
     """Exposes a raw device pointer through __cuda_array_interface__ so torch can wrap it without a copy."""
 
@@ -112,8 +121,12 @@ class VecWorld:
                  device: int | str | torch.device = 0, reward_dim: int = 1, walkable_lasers: bool = True, auto_reset: bool = True,
                  lle_semantics: bool = True, write_obs: bool = True, seed: int = 0, env_id_base: int = 0,
                  extras: str | Sequence[int] | None = None, pbrs: dict | None = None, obs_type: str = "layered",
-                 padding_size: int = 0, randomize_lasers: bool = False, state_type: str = "state", episode_stats: bool = False):
+                 padding_size: int = 0, randomize_lasers: bool = False, state_type: str = "state", episode_stats: bool = False,
+                 obs_dtype: torch.dtype | str = torch.float32):
         """obs_type: an ObservationType value (observations.py:37-60) other than "rgb-image"; padding_size for "layered-padded".
+        obs_dtype: torch.float32 (default) or torch.int8 (also "float32" / "int8"): the element type of `obs`.  Every value of a
+        layered, padded, flattened or perspective observation is -1, 0 or 1, so int8 holds the same observation in a quarter of the
+        HBM bytes (`obs.to(torch.bfloat16)` and `obs.float()` are exact).  Partial and state observations are float32 only.
         state_type: the ObservationType whose first-agent observation is the state (Builder.state_type, builder.py:51-58).
         extras: None | "laser_subgoal" (all sources) | source indices (World::sources() order) — Builder.add_extras.
         pbrs: None | dict(gamma=0.99, reward_value=0.5, lasers_to_reward=None | indices, with_extras=True) — Builder.pbrs
@@ -134,6 +147,8 @@ class VecWorld:
         opts.obs_type, opts.obs_param, self._flatten = obs_spec(obs_type, padding_size)
         opts.randomize_lasers = int(bool(randomize_lasers))
         opts.episode_stats = int(bool(episode_stats))
+        self.obs_dtype = _obs_dtype(obs_dtype)
+        opts.obs_dtype = _native.DTYPE_I8 if self.obs_dtype == torch.int8 else _native.DTYPE_F32
         self.state_type = getattr(state_type, "value", state_type)
         opts.state_type, opts.state_param, self._state_flatten = obs_spec(state_type, 0)  # the reference builds it with padding_size = 0 (env.py:86)
         extras_src = None if extras in (None, "laser_subgoal") else [int(x) for x in extras]
@@ -185,7 +200,7 @@ class VecWorld:
         self.obs_invalid = bool(b.obs_invalid)
         self.obs_shape = (b.obs_c,) if self.obs_kind == OBS_STATE else (b.obs_c, b.obs_h, b.obs_w)  # one agent's observation
         if write_obs:
-            rows = wrap(b.obs, (N, self.obs_stride), "<f4")
+            rows = wrap(b.obs_i8, (N, self.obs_stride), "|i1") if int(b.obs_dtype) == _native.DTYPE_I8 else wrap(b.obs, (N, self.obs_stride), "<f4")
             block = self.obs_shape if self.obs_view_agents else (A, *self.obs_shape)
             n = int(np.prod(block))
             self.obs = rows[:, :n].unflatten(1, block)

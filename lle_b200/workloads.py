@@ -139,8 +139,9 @@ class Workload:
 def algorithmic_bytes(vec: VecWorld) -> dict:
     """SURVEY.md §8(d): B = OBS + ST + AV + AC + RDE + 2*S for one env-step of `vec`; OBS = the block `vec.obs` holds per env."""
     A, G, R = vec.n_agents, vec.n_gems, vec.reward_dim
-    # the floats the observation generator materialises per env (layered / state: one copy viewed by every agent)
-    obs = 4 * int(np.prod(vec.obs.shape[1:])) if vec.obs is not None else 0
+    # the elements the observation generator materialises per env (layered / state: one copy viewed by every agent), at the
+    # vec's element size (4 bytes, or 1 for obs_dtype=torch.int8)
+    obs = vec.obs.element_size() * int(np.prod(vec.obs.shape[1:])) if vec.obs is not None else 0
     st, av, ac = 4 * (3 * A + G), 5 * A, A
     rde = 4 * R + 1 + A + 1  # reward, done, events, err
     return dict(obs=obs, state=st, avail=av, actions=ac, reward_done_events=rde, record_rw=2 * vec.record_bytes,
