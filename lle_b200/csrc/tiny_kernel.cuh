@@ -80,16 +80,7 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 4 : LLE_TINY_MIN_CTAS) lle
     const LleCellBeams** sbeams = reinterpret_cast<const LleCellBeams**>(smeta + 32);  // PARTIAL: [32] the beam table of lane l's map
     const int E = p.E;
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    if (p.in_flag) {  // host-supplied actions still in flight on the copy stream
-        if (lane == 0)
-            while (!sys_flag_ready(p.in_flag, p.in_need)) __nanosleep(100);
-        __syncwarp();
-    }
-    if (p.sched_check) {
-        if (lane == 0)
-            while (!sched_slot_armed(p.sched + 2, p.sched_gen)) __nanosleep(32);
-        __syncwarp();
-    }
+    launch_wait(p, lane);
 
     const uint32_t n_pairs = p.n_tickets * (uint32_t)p.n_steps;
     const bool single_step = p.n_steps == 1;
@@ -103,34 +94,14 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 4 : LLE_TINY_MIN_CTAS) lle
 
     // The next (step, ticket) pair is taken, its flag looked at and its records and map index requested while this ticket's
     // observation is rendered: the latencies of a ticket's first loads hide behind the previous ticket's stores.
-    uint32_t next_in_chunk = 0;
     bool have_next = false, next_ready = false;
     uint32_t next_pair = 0;
     int next_map = 0;
-    // pairs are taken `chunk` at a time: one atomic on the launch's counter per chunk (same-address atomics are serialised by
-    // the L2: one per ticket of 32 tiny worlds is what bounded this kernel at 8.4 ns per ticket, whatever the SM side did)
-    const uint32_t chunk = (uint32_t)max(p.ticket_chunk, 1);
-    uint32_t chunk_end = 0;  // one past the last pair of the chunk this warp holds
     const uint32_t warp_global = blockIdx.x * kWarps + warp;
-    // On an idle device (the host saw every earlier launch retire: a closed loop) all CTAs are resident at once and a warp's first
-    // pair is its own index - no round trip to the launch's counter before it can start.  Not when launches overlap: CTAs then
-    // trickle in as their predecessors' retire, and a pair pinned to a late CTA would hold up everything behind it.
-    bool first_pair = p.sched_check == 0;
-    auto take_pair = [&]() -> uint32_t {  // lane 0 only
-        if (first_pair) {
-            first_pair = false;
-            return warp_global;
-        }
-        if (chunk_end == 0 || next_in_chunk >= chunk_end) {
-            next_in_chunk = (p.sched_check == 0 ? p.n_warps_total : 0u) + atomicAdd(&p.sched[0], chunk);  // behind the static pairs, if any
-            chunk_end = next_in_chunk + chunk;
-        }
-        return next_in_chunk++;
-    };
     for (;;) {
         uint32_t pair = next_pair;
-        if (!have_next) {
-            if (lane == 0) pair = take_pair();
+        if (!have_next) {  // the first pair
+            if (lane == 0) pair = take_pair(p, true, warp_global);
             pair = __shfl_sync(kFull, pair, 0);
         }
         if (pair >= n_pairs) break;
@@ -271,7 +242,7 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 4 : LLE_TINY_MIN_CTAS) lle
             uint32_t np2 = 0;
             int rdy = 0;
             if (lane == 0) {
-                np2 = take_pair();
+                np2 = take_pair(p, false, warp_global);
                 if (np2 < n_pairs) rdy = ticket_ready(p.flags + (single_step ? np2 : np2 % p.n_tickets), p.seq + (single_step ? 0u : np2 / p.n_tickets) - 1u) ? 1 : 0;
             }
             next_pair = __shfl_sync(kFull, np2, 0);

@@ -31,6 +31,8 @@ int fail(int code, const std::string& msg) { g_error = msg; return code; }
                         std::string(#expr) + ": " + cudaGetErrorString(_e));                               \
     } while (0)
 
+using KernelFn = void (*)(KParams);  // every instantiation of lle_world_kernel and lle_tiny_step_kernel
+
 }  // namespace lle
 
 using namespace lle;
@@ -100,19 +102,18 @@ struct lle_vec {
     bool fast = false, pdl = true;
     int feature_limit = 0;
     bool by_feature = false;  // partial observations rendered feature by feature (kernel KIND 2): every map has <= 2 s^2 features
-    bool force_narrow = false;  // LLE_B200_FORCE_NARROW=1 (tests)
     // tiny maps: step launches run the thread-per-world kernel (tiny_kernel.cuh) with its own tiling and grid
     bool tiny = false, tiny_partial = false;
-    int tiny_E = 8, tiny_warp_smem = 0, tiny_grid = 0, tiny_chunk = 1;
-    int chunk = 1;  // general kernel: pairs per scheduler atomic (LLE_B200_CHUNK)
+    int tiny_E = 8, tiny_warp_smem = 0, tiny_grid = 0;
     size_t tiny_smem = 0;
+    // the instantiations this vec launches (select_kernels): step, step of a parts loop, reset, set_state, tiny step (or null)
+    KernelFn k_step = nullptr, k_step_parts = nullptr, k_reset = nullptr, k_set_state = nullptr, k_tiny = nullptr;
     uint32_t* h_retired_seq = nullptr;  // pinned, device-mapped: [0] sequence number of the last step launch that retired,
                                         // [32] number of launches of this vec (any mode) whose last warp has left
     uint32_t* d_retired_count = nullptr;  // device counter behind [32]
     MapDev map0;                        // the tables of map 0 as device pointers (kernel parameter of single-map batches)
     bool has_map0 = false;
     bool narrow_next = false;  // the next step launch finds its predecessor still running: use the narrow grid
-    int narrow_depth = 1;      // step launches in flight from which the narrow grid is used (LLE_B200_NARROW_DEPTH)
     int grid = 0, grid_step = 0, grid_idle = 0, Wd = 32, group = 4, E = 1, n_chunks = 1, chunk_floats = 0, tile_floats = 0, n_buf = 1, warp_smem = 0;
     size_t smem = 0;
     uint64_t t = 0, launches = 0;
@@ -155,48 +156,43 @@ namespace {
 constexpr int kSchedSlots = 8;
 constexpr int kSchedSlotWords = 32;
 
-// The thread-per-world step kernel of a vec with A agents (tiny_kernel.cuh): one instantiation per agent count and element type
-template <typename OT>
-cudaError_t launch_tiny(const lle_vec* v, const cudaLaunchConfig_t& cfg, const KParams& p) {
-    if constexpr (sizeof(OT) == 4) {
-        switch (v->A * 2 + (v->tiny_partial ? 1 : 0)) {
-            case 2: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<1, false>, p);
-            case 3: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<1, true>, p);
-            case 4: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<2, false>, p);
-            case 5: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<2, true>, p);
-            case 6: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<3, false>, p);
-            case 7: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<3, true>, p);
-            case 8: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<4, false>, p);
-            default: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<4, true>, p);
-        }
-    } else {  // partial observations are float only
-        switch (v->A) {
-            case 1: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<1, false, OT>, p);
-            case 2: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<2, false, OT>, p);
-            case 3: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<3, false, OT>, p);
-            default: return cudaLaunchKernelEx(&cfg, lle_tiny_step_kernel<4, false, OT>, p);
-        }
-    }
+// The kernels a vec launches: the one place that names an instantiation of lle_world_kernel or lle_tiny_step_kernel.
+// KIND 1 (FAST) for the common layered shape, KIND 2 (the feature-driven renderer) for partial observations of sparse maps, KIND 0
+// for everything else; a parts loop has its own step instantiations.  Partial observations are float only: no int8 KIND 2 or
+// PARTIAL tiny kernel.  The thread-per-world step kernel (tiny_kernel.cuh) has one instantiation per agent count.
+void select_kernels(lle_vec* v) {
+    auto world = [v](KernelFn step, KernelFn step_parts, KernelFn reset, KernelFn set_state) {
+        v->k_step = step;
+        v->k_step_parts = step_parts;
+        v->k_reset = reset;
+        v->k_set_state = set_state;
+    };
+    if (v->i8 && v->fast)
+        world(lle_world_kernel<MODE_STEP, 1, false, int8_t>, lle_world_kernel<MODE_STEP, 1, true, int8_t>,
+              lle_world_kernel<MODE_RESET, 1, false, int8_t>, lle_world_kernel<MODE_SET_STATE, 1, false, int8_t>);
+    else if (v->i8)
+        world(lle_world_kernel<MODE_STEP, 0, false, int8_t>, lle_world_kernel<MODE_STEP, 0, true, int8_t>,
+              lle_world_kernel<MODE_RESET, 0, false, int8_t>, lle_world_kernel<MODE_SET_STATE, 0, false, int8_t>);
+    else if (v->fast)
+        world(lle_world_kernel<MODE_STEP, 1>, lle_world_kernel<MODE_STEP, 1, true>, lle_world_kernel<MODE_RESET, 1>,
+              lle_world_kernel<MODE_SET_STATE, 1>);
+    else if (v->by_feature)
+        world(lle_world_kernel<MODE_STEP, 2>, lle_world_kernel<MODE_STEP, 2, true>, lle_world_kernel<MODE_RESET, 2>,
+              lle_world_kernel<MODE_SET_STATE, 2>);
+    else
+        world(lle_world_kernel<MODE_STEP, 0>, lle_world_kernel<MODE_STEP, 0, true>, lle_world_kernel<MODE_RESET, 0>,
+              lle_world_kernel<MODE_SET_STATE, 0>);
+    static const KernelFn tiny[3][4] = {  // [float / float PARTIAL / int8][A - 1]
+        {lle_tiny_step_kernel<1>, lle_tiny_step_kernel<2>, lle_tiny_step_kernel<3>, lle_tiny_step_kernel<4>},
+        {lle_tiny_step_kernel<1, true>, lle_tiny_step_kernel<2, true>, lle_tiny_step_kernel<3, true>, lle_tiny_step_kernel<4, true>},
+        {lle_tiny_step_kernel<1, false, int8_t>, lle_tiny_step_kernel<2, false, int8_t>, lle_tiny_step_kernel<3, false, int8_t>,
+         lle_tiny_step_kernel<4, false, int8_t>},
+    };
+    v->k_tiny = v->tiny ? tiny[v->i8 ? 2 : v->tiny_partial ? 1 : 0][std::min(v->A, 4) - 1] : nullptr;
 }
 
-template <int MODE, typename OT>
-cudaError_t launch_world(const lle_vec* v, const cudaLaunchConfig_t& cfg, const KParams& p) {
-    if constexpr (MODE == MODE_STEP) {
-        if (p.part_in) {  // a parts loop: its own instantiations
-            if (v->fast) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 1, true, OT>, p);
-            if constexpr (sizeof(OT) == 4)
-                if (v->by_feature) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 2, true>, p);
-            return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE_STEP, 0, true, OT>, p);
-        }
-    }
-    if (v->fast) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 1, false, OT>, p);
-    if constexpr (sizeof(OT) == 4)  // the feature-driven renderer draws partial observations: float only
-        if (v->by_feature) return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 2>, p);
-    return cudaLaunchKernelEx(&cfg, lle_world_kernel<MODE, 0, false, OT>, p);
-}
-
-template <int MODE>
 cudaError_t launch_mode(lle_vec* v, KParams& p, cudaStream_t s) {
+    const bool step = p.mode == MODE_STEP;
     // Programmatic stream serialization: the kernel calls griddepcontrol.wait before it touches anything a
     // previous launch wrote, so its prologue may overlap the tail of the launch before it.
     cudaLaunchConfig_t cfg;
@@ -204,13 +200,13 @@ cudaError_t launch_mode(lle_vec* v, KParams& p, cudaStream_t s) {
     // A single step that may overlap its predecessor runs on a narrow grid (grid_step CTAs), so that several consecutive
     // step launches are resident at once and form a software pipeline over the epoch flags: while step t drains, steps
     // t+1.. already stream their first tickets.  Rollouts, resets and set_state use the full-width grid.
-    const bool overlaps = v->pdl && MODE == MODE_STEP && v->last_was_step && v->last_stream == s;
+    const bool overlaps = v->pdl && step && v->last_was_step && v->last_stream == s;
     // (A parts loop takes the full grid too: its launches wait for the host part by part, and a wide grid keeps enough unblocked
     // warps resident.  Level 6 x 65,536, 8 parts, us per step with 2 / 3 / 5 CTAs per SM: 96.9 / 87.8 / 84.5.)
     // A single step that finds the device idle takes four CTAs per SM of the five, which leaves room for the first CTAs of the
     // launch that follows it (the driver's 20-step window after a sync, idle launch at 5 / 4 / 3 / 2 CTAs per SM: 79.8 / 78.7 /
     // 78.8 / 78.9 us per step).
-    const int grid = (MODE == MODE_STEP && p.n_steps == 1 && !p.part_in) ? ((overlaps && v->narrow_next) ? v->grid_step : v->grid_idle) : v->grid;
+    const int grid = (step && p.n_steps == 1 && !p.part_in) ? ((overlaps && v->narrow_next) ? v->grid_step : v->grid_idle) : v->grid;
     v->narrow_next = false;
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3(kThreads);
@@ -223,19 +219,17 @@ cudaError_t launch_mode(lle_vec* v, KParams& p, cudaStream_t s) {
     attr[0].val.programmaticStreamSerializationAllowed = overlaps ? 1 : 0;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if constexpr (MODE == MODE_STEP) {
-        if (v->tiny && !p.part_in) {  // thread-per-world kernel: same tickets, flags and records, its own tile layout (not in a parts loop)
-            cfg.gridDim = dim3((unsigned)v->tiny_grid);
-            cfg.dynamicSmemBytes = v->tiny_smem;
-            p.n_warps_total = (uint32_t)(v->tiny_grid * kWarps);
-            p.E = v->tiny_E;
-            p.tile_floats = (int32_t)(v->tiny_E * v->obs_stride);
-            p.warp_smem_bytes = v->tiny_warp_smem;
-            p.ticket_chunk = v->tiny_chunk;
-            return v->i8 ? launch_tiny<int8_t>(v, cfg, p) : launch_tiny<float>(v, cfg, p);
-        }
+    KernelFn kern = step ? (p.part_in ? v->k_step_parts : v->k_step) : p.mode == MODE_RESET ? v->k_reset : v->k_set_state;
+    if (step && v->tiny && !p.part_in) {  // thread-per-world kernel: same tickets, flags and records, its own tile layout (not in a parts loop)
+        kern = v->k_tiny;
+        cfg.gridDim = dim3((unsigned)v->tiny_grid);
+        cfg.dynamicSmemBytes = v->tiny_smem;
+        p.n_warps_total = (uint32_t)(v->tiny_grid * kWarps);
+        p.E = v->tiny_E;
+        p.tile_floats = (int32_t)(v->tiny_E * v->obs_stride);
+        p.warp_smem_bytes = v->tiny_warp_smem;
     }
-    return v->i8 ? launch_world<MODE, int8_t>(v, cfg, p) : launch_world<MODE, float>(v, cfg, p);
+    return cudaLaunchKernelEx(&cfg, kern, p);
 }
 // Host bookkeeping (launch index, sequence number, "the last launch was a step") advances only when the launch was accepted.
 cudaError_t launch(lle_vec* v, KParams& p, cudaStream_t s) {
@@ -259,16 +253,15 @@ cudaError_t launch(lle_vec* v, KParams& p, cudaStream_t s) {
             // (synchronous stepping, a policy between two steps) takes the full-width grid: alone, a narrow launch cannot
             // saturate HBM.  Measured on B200, level 6 x 65,536, us/step in windows of 20 / 2,000 launches after a sync, CTAs per
             // SM 1 / 2 / 3 / 5: 81.6 / 79.4 / 80.6 / 83.6 and 75.6 / 76.3 / 78.6 / 82.3 (profiles/grid_sweep_r02.jsonl).
-            v->narrow_next = v->force_narrow || (int32_t)(v->seq - *(volatile uint32_t*)v->h_retired_seq) >= v->narrow_depth;
-            e = launch_mode<MODE_STEP>(v, p, s);
+            v->narrow_next = (int32_t)(v->seq - *(volatile uint32_t*)v->h_retired_seq) >= 1;
+            e = launch_mode(v, p, s);
             if (e != cudaSuccess) return e;
             v->launch_index++;
             v->seq += (uint32_t)p.n_steps;
             v->last_was_step = true;
             v->last_stream = s;
             return e;
-        case MODE_RESET: e = launch_mode<MODE_RESET>(v, p, s); break;
-        default: e = launch_mode<MODE_SET_STATE>(v, p, s); break;
+        default: e = launch_mode(v, p, s); break;
     }
     if (e != cudaSuccess) return e;
     v->launch_index++;
@@ -309,9 +302,9 @@ cudaError_t smem_optin(int device, int* out) {
     return cudaSuccess;
 }
 
-template <int MODE, int KIND, bool PARTS = false, typename OT = float>
-cudaError_t configure_kernel(size_t smem, int* blocks) {
-    auto kern = lle_world_kernel<MODE, KIND, PARTS, OT>;
+// Raises the kernel's dynamic shared-memory limit to the opt-in maximum and lowers *blocks (< 0: not set yet) to the CTAs per SM
+// it reaches with `smem` bytes each
+cudaError_t configure_kernel(KernelFn kern, size_t smem, int* blocks) {
     int dev = 0, optin = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = smem_optin(dev, &optin);
@@ -374,7 +367,6 @@ KParams base_params(lle_vec* v) {
     p.n_tickets = (uint32_t)(v->N_pad / v->group);
     p.n_warps_total = (uint32_t)(v->grid * kWarps);
     p.n_steps = 1;
-    p.ticket_chunk = v->chunk;
     p.extras = v->d_extras; p.JE = v->JE; p.pbrs_on = v->opts.pbrs ? 1 : 0;
     p.extras_set = v->extras_set; p.pbrs_set = v->pbrs_set;
     p.pbrs_gamma = v->opts.pbrs_gamma; p.pbrs_value = v->opts.pbrs_reward_value;
@@ -696,7 +688,7 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
     // tiny observations: the logic dominates, pack more worlds per pass.  In bytes: a level-6 int8 row (1,872 B) is small and
     // runs on the thread-per-world kernel (level 6 x 65,536 on one B200: 45.5 us per step there, 65.9 on the fast kernel)
     const bool small_obs = v->obs_stride * es < 2048;
-    v->Wd = std::max(v->Wd, std::min(32, env_int("LLE_B200_MIN_WD", small_obs ? 1 : 2)));
+    v->Wd = std::max(v->Wd, small_obs ? 1 : 2);
     const int64_t stride = v->obs_stride;
     // 4-8 KB per bulk store; partial observations: up to 9.6 KB, one tile buffer and 16 worlds per ticket, which keeps five
     // CTAs per SM (sweep of buffers x tile size x ticket size on level 6 x 65,536, us per step before -> after:
@@ -713,7 +705,7 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
     // long as one ticket, so larger windows (more rounds per ticket) stay on the general kernel, which has four times the warps.
     const bool tiny_partial = partial_obs && tiny_record && (stride * 4 < 2048 || env_int("LLE_B200_TINY_PARTIAL", 0));
     // (targets and limits in 4-byte units, as measured on f32; elements of the vec's type below)
-    const int64_t kTileTargetFloats = env_int("LLE_B200_TILE_TARGET", partial_obs ? 2400 : small_obs ? 2048 : 1024) * 4 / es;
+    const int64_t kTileTargetFloats = (partial_obs ? 2400 : small_obs ? 2048 : 1024) * 4 / es;
     // the partial renderer builds whole worlds (all agents' windows) in one tile: allow up to 48 KB per warp
     const int64_t kTileMaxFloats = (spec.kind == LLE_OBS_PARTIAL ? 12288 : 6144) * 4 / es;
     if (spec.kind == LLE_OBS_PARTIAL && stride > kTileMaxFloats)
@@ -740,10 +732,6 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         while (v->group > std::max(8, 32 / v->Wd) && (v->N_pad / v->group < 2048 || (int64_t)v->group * stride * es > (6 << 20))) v->group >>= 1;
         v->n_buf = 2;
     }
-    {
-        int g = env_int("LLE_B200_GROUP", v->group);
-        if (g >= v->E && g >= 32 / v->Wd && g <= 32 && (g & (g - 1)) == 0) v->group = g;
-    }
     auto warp_smem_for = [&](int n_buf) {
         size_t bytes = (size_t)n_buf * v->tile_floats * es;            // tiles
         bytes += (size_t)v->group * v->L.stride * 4;                   // records of the group
@@ -751,55 +739,26 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
         bytes += (size_t)(2 * n_buf * v->E + n_buf + v->group) * 4;    // tags + map ids + fresh flags
         return (int)((bytes + 127) / 128 * 128);
     };
-    v->n_buf = std::max(1, std::min(2, env_int("LLE_B200_NBUF", v->n_buf)));          // tuning knobs (development)
     v->warp_smem = warp_smem_for(v->n_buf);
     v->smem = (size_t)v->warp_smem * kWarps;
-    v->pdl = env_int("LLE_B200_PDL", 1) != 0;
-    v->force_narrow = env_int("LLE_B200_FORCE_NARROW", 0) != 0;
-    v->narrow_depth = std::max(1, env_int("LLE_B200_NARROW_DEPTH", 1));
-    v->chunk = std::max(1, std::min(64, env_int("LLE_B200_CHUNK", 1)));
     int max_patch = 0;
     for (int k = 0; k < n_maps; ++k) max_patch = std::max(max_patch, (int)cms[k]->header().n_patch);
     for (const auto& m : v->variant_maps) max_patch = std::max(max_patch, (int)m.header().n_patch);
-    v->fast = v->n_chunks == 1 && v->E <= 32 && v->n_buf == 1 && max_patch <= 64 && v->L.stride <= 32 && opts->write_obs &&
-              spec.kind == LLE_OBS_LAYERED && !v->randomize && !random_starts && !env_int("LLE_B200_NO_FAST", 0);
-    if (spec.kind == LLE_OBS_PARTIAL && !env_int("LLE_B200_NO_FEATURES", 0)) {
+    v->fast = v->n_chunks == 1 && v->n_buf == 1 && max_patch <= 64 && v->L.stride <= 32 && opts->write_obs &&
+              spec.kind == LLE_OBS_LAYERED && !v->randomize && !random_starts;
+    if (spec.kind == LLE_OBS_PARTIAL) {
         v->by_feature = true;  // a window task costs about three feature tasks (measured on level 6)
-        v->feature_limit = env_int("LLE_B200_FEATURE_FACTOR", 2) * spec.param * spec.param;
+        v->feature_limit = 2 * spec.param * spec.param;
         for (int k = 0; k < n_maps; ++k) v->by_feature = v->by_feature && (int)cms[k]->header().n_patch <= v->feature_limit;
         for (const auto& m : v->variant_maps) v->by_feature = v->by_feature && (int)m.header().n_patch <= v->feature_limit;
     }
-    int blocks_per_sm = -1;  // the grid is shared by the three modes: size it for the most demanding one
-    if (v->i8 && v->fast) {
-        LLE_CUDA((configure_kernel<MODE_STEP, 1, false, int8_t>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_STEP, 1, true, int8_t>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_RESET, 1, false, int8_t>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_SET_STATE, 1, false, int8_t>(v->smem, &blocks_per_sm)));
-    } else if (v->i8) {
-        LLE_CUDA((configure_kernel<MODE_STEP, 0, false, int8_t>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_STEP, 0, true, int8_t>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_RESET, 0, false, int8_t>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_SET_STATE, 0, false, int8_t>(v->smem, &blocks_per_sm)));
-    } else if (v->fast) {
-        LLE_CUDA((configure_kernel<MODE_STEP, 1>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_STEP, 1, true>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_RESET, 1>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_SET_STATE, 1>(v->smem, &blocks_per_sm)));
-    } else if (v->by_feature) {
-        LLE_CUDA((configure_kernel<MODE_STEP, 2>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_STEP, 2, true>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_RESET, 2>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_SET_STATE, 2>(v->smem, &blocks_per_sm)));
-    } else {
-        LLE_CUDA((configure_kernel<MODE_STEP, 0>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_STEP, 0, true>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_RESET, 0>(v->smem, &blocks_per_sm)));
-        LLE_CUDA((configure_kernel<MODE_SET_STATE, 0>(v->smem, &blocks_per_sm)));
-    }
-    if (blocks_per_sm < 1) return fail(LLE_CUDA_ERROR, "kernel does not fit on an SM");
     // Tiny maps (small observation, few agents, a record of at most 8 words): the step runs one thread per world.
     v->tiny = ((v->fast && small_obs) || tiny_partial) && tiny_record && v->group == 32;
     v->tiny_partial = v->tiny && tiny_partial;
+    select_kernels(v.get());
+    int blocks_per_sm = -1;  // the grid is shared by the three modes: size it for the most demanding one
+    for (KernelFn k : {v->k_step, v->k_step_parts, v->k_reset, v->k_set_state}) LLE_CUDA(configure_kernel(k, v->smem, &blocks_per_sm));
+    if (blocks_per_sm < 1) return fail(LLE_CUDA_ERROR, "kernel does not fit on an SM");
     if (v->tiny) {
         // worlds per tile / bulk store (measured on 2^20 5x5 worlds, us per step: 4: 232, 8: 243, 16: 343, 32: 558 - occupancy)
         int e_default = 4;
@@ -811,65 +770,35 @@ int lle_vec_create(const lle_map* const* maps, int32_t n_maps, const int32_t* ma
             e_default = 1;
             while (e_default < 32 && 2 * e_default * stride * 4 <= 13312) e_default *= 2;
         }
-        int e = env_int("LLE_B200_TINY_E", e_default);
-        v->tiny_E = (e >= (tiny_partial ? 1 : 4) && e <= 32 && (e & (e - 1)) == 0) ? e : e_default;
+        v->tiny_E = e_default;
         auto tiny_bytes = [&]() {  // the records' columns + the prefetched next records, list pointers, list lengths, the tile
             const size_t bytes = 2 * (size_t)v->L.stride * 32 * 4 + 32 * 8 + 32 * 4 + (tiny_partial ? 32 * 8 : 0) + (size_t)v->tiny_E * stride * es;
             return (bytes + 127) / 128 * 128;
         };
-        v->tiny_chunk = std::max(1, std::min(64, env_int("LLE_B200_TINY_CHUNK", 1)));
         v->tiny_warp_smem = (int)tiny_bytes();
         v->tiny_smem = (size_t)v->tiny_warp_smem * kWarps;
-        int tb = 0;
-        auto configure = [&](auto kern) -> cudaError_t {
-            int optin = 0;
-            cudaError_t e2 = smem_optin(v->device, &optin);
-            if (e2 == cudaSuccess && v->tiny_smem > (size_t)optin) return cudaErrorInvalidValue;
-            if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, optin);
-            if (e2 != cudaSuccess) return e2;
-            return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tb, kern, kThreads, v->tiny_smem);
-        };
-        if (v->i8) {
-            switch (v->A) {
-                case 1: LLE_CUDA(configure(lle_tiny_step_kernel<1, false, int8_t>)); break;
-                case 2: LLE_CUDA(configure(lle_tiny_step_kernel<2, false, int8_t>)); break;
-                case 3: LLE_CUDA(configure(lle_tiny_step_kernel<3, false, int8_t>)); break;
-                default: LLE_CUDA(configure(lle_tiny_step_kernel<4, false, int8_t>)); break;
-            }
-        } else switch (v->A * 2 + (tiny_partial ? 1 : 0)) {
-            case 2: LLE_CUDA(configure(lle_tiny_step_kernel<1, false>)); break;
-            case 3: LLE_CUDA(configure(lle_tiny_step_kernel<1, true>)); break;
-            case 4: LLE_CUDA(configure(lle_tiny_step_kernel<2, false>)); break;
-            case 5: LLE_CUDA(configure(lle_tiny_step_kernel<2, true>)); break;
-            case 6: LLE_CUDA(configure(lle_tiny_step_kernel<3, false>)); break;
-            case 7: LLE_CUDA(configure(lle_tiny_step_kernel<3, true>)); break;
-            case 8: LLE_CUDA(configure(lle_tiny_step_kernel<4, false>)); break;
-            default: LLE_CUDA(configure(lle_tiny_step_kernel<4, true>)); break;
+        int tb = -1;
+        LLE_CUDA(configure_kernel(v->k_tiny, v->tiny_smem, &tb));
+        if (tb < 1) {
+            v->tiny = false;
+            v->k_tiny = nullptr;
         }
-        if (tb < 1) v->tiny = false;
-        tb = std::min(tb, std::max(1, env_int("LLE_B200_TINY_CTAS_PER_SM", 16)));
         const int64_t tickets = v->N_pad / v->group;
         v->tiny_grid = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)prop.multiProcessorCount * tb, (tickets + kWarps - 1) / kWarps));
     }
-    blocks_per_sm = std::min(blocks_per_sm, std::max(1, env_int("LLE_B200_MAX_CTAS_PER_SM", 16)));
     const int64_t n_tickets = v->N_pad / v->group;
     v->grid = (int)std::min<int64_t>((int64_t)prop.multiProcessorCount * blocks_per_sm, (n_tickets + kWarps - 1) / kWarps);
     v->grid = std::max(v->grid, 1);
     {
         // measured on B200 (us/step, 1 CTA per SM vs the full grid): level 6 x 65,536: 76.5 vs 81.4; level 1: 49.7 vs 54.0;
         // 1,024 generated 5x5 maps x 1,024 (instruction-bound, 445 us steps): 467 vs 445 -> tiny observations keep the full grid
-        const int step_ctas = std::max(1, std::min(blocks_per_sm, env_int("LLE_B200_STEP_CTAS_PER_SM", small_obs ? blocks_per_sm : 2)));
+        const int step_ctas = small_obs ? blocks_per_sm : std::min(blocks_per_sm, 2);
         v->grid_step = (int)std::min<int64_t>((int64_t)prop.multiProcessorCount * step_ctas, (n_tickets + kWarps - 1) / kWarps);
         v->grid_step = std::max(v->grid_step, 1);
     }
     {
-        const int idle_ctas = std::max(1, std::min(blocks_per_sm, env_int("LLE_B200_IDLE_CTAS_PER_SM", small_obs ? blocks_per_sm : 4)));
+        const int idle_ctas = small_obs ? blocks_per_sm : std::min(blocks_per_sm, 4);
         v->grid_idle = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)prop.multiProcessorCount * idle_ctas, (n_tickets + kWarps - 1) / kWarps));
-    }
-    if (const int cap = env_int("LLE_B200_GRID_CAP", 0); cap > 0) {  // development: CTAs per launch (several vecs sharing one GPU)
-        v->grid = std::min(v->grid, cap);
-        v->grid_step = std::min(v->grid_step, cap);
-        v->grid_idle = std::min(v->grid_idle, cap);
     }
 
     // ---- device memory

@@ -118,7 +118,6 @@ struct KParams {
     uint32_t n_tickets, n_warps_total;
     uint64_t* timeline;    // development aid: per warp {start, first store, last store, end} in ns (globaltimer), or nullptr
     int32_t n_steps;       // steps in this launch (> 1: rollout with device-sampled actions)
-    int32_t ticket_chunk;  // tiny-map kernel: consecutive (step, ticket) pairs a warp takes with one atomic (the L2 serialises same-address atomics)
     // LaserSubgoal extras / PotentialShapedLLE
     float* extras;         // [N_pad][A][JE] or nullptr
     int32_t JE, pbrs_on;
@@ -740,6 +739,31 @@ __device__ __forceinline__ bool sched_slot_armed(const uint32_t* gen, uint32_t w
     asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(gen) : "memory");
     return v == want;
 }
+// What a launch waits for before it takes its first pair.  Host-supplied actions still in flight on the copy stream (independent
+// of this stream: no cycle).  And its scheduler slot: slots rotate over the launches, and programmatic dependent launch lets many
+// small launches be resident at once, so the launch that used this slot kSchedSlots launches ago may still be running: wait until
+// its last warp has re-armed the slot (it never waits for us, and all of its CTAs are resident by the time this launch may start:
+// no cycle).
+__device__ __forceinline__ void launch_wait(const KParams& p, int lane) {
+    if (p.in_flag) {
+        if (lane == 0)
+            while (!sys_flag_ready(p.in_flag, p.in_need)) __nanosleep(100);
+        __syncwarp();
+    }
+    if (p.sched_check) {
+        if (lane == 0)
+            while (!sched_slot_armed(p.sched + 2, p.sched_gen)) __nanosleep(32);
+        __syncwarp();
+    }
+}
+// Lane 0: the warp's next (step, ticket) pair (`first`: its first one).  On an idle device (the host saw every earlier launch
+// retire: a closed loop) all CTAs are resident at once and a warp's first pair is its own index - no round trip to the launch's
+// counter before it can start.  Not when launches overlap: CTAs then trickle in as their predecessors retire, and a pair pinned to
+// a late CTA would hold up everything behind it.
+__device__ __forceinline__ uint32_t take_pair(const KParams& p, bool first, uint32_t warp_global) {
+    if (p.sched_check == 0) return first ? warp_global : p.n_warps_total + atomicAdd(&p.sched[0], 1u);  // behind the static pairs
+    return atomicAdd(&p.sched[0], 1u);
+}
 template <int N>
 __device__ __forceinline__ void bulk_wait() { asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory"); }
 
@@ -888,51 +912,22 @@ __global__ void __launch_bounds__(kThreads, LLE_MIN_CTAS) lle_world_kernel(const
     // Reset / set_state wait for the whole previous launch.  A step does not: it orders itself ticket by ticket with
     // the epoch flags, so its first tickets start while the previous step's last ones are still draining.
     if constexpr (MODE != MODE_STEP) asm volatile("griddepcontrol.wait;" ::: "memory");
-
-    if constexpr (MODE == MODE_STEP) {
-        if (p.in_flag) {  // host-supplied actions still in flight on the copy stream (independent of this stream: no cycle)
-            if (lane == 0)
-                while (!sys_flag_ready(p.in_flag, p.in_need)) __nanosleep(100);
-            __syncwarp();
-        }
-    }
+    launch_wait(p, lane);
     const uint32_t warp_global = blockIdx.x * kWarps + warp;
     const uint32_t n_pairs = p.n_tickets * (uint32_t)p.n_steps;  // (step, ticket) pairs, handed out in order (the host keeps it < 2^31)
-    // Scheduler slots rotate over the launches.  Programmatic dependent launch lets many small launches be resident at once,
-    // so the launch that used this slot kSchedSlots launches ago may still be running: wait until its last warp has re-armed
-    // the slot (it never waits for us, and all of its CTAs are resident by the time this launch may start: no cycle).
-    if (p.sched_check) {
-        if (lane == 0)
-            while (!sched_slot_armed(p.sched + 2, p.sched_gen)) __nanosleep(32);
-        __syncwarp();
-    }
     uint64_t t_first = 0, t_last = 0;
     if (p.timeline && lane == 0) p.timeline[warp_global * 4] = globaltimer_ns();
     int step_index = 0;
     bool first = true;
     uint32_t owed_ticket = 0, owed_seq = 0;  // the previous ticket, whose completion is published once its stores are done
     bool owed = false;
-    // pairs are taken `ticket_chunk` at a time with one atomic on the launch's counter (the L2 serialises same-address atomics)
-    const uint32_t chunk = (uint32_t)max(p.ticket_chunk, 1);
-    uint32_t chunk_next = 0, chunk_end = 0;  // lane 0: the pairs of the chunk this warp holds
     const bool single_step = p.n_steps == 1;
-    // On an idle device (the host saw every earlier launch retire: a closed loop) all CTAs are resident at once and a warp's first
-    // pair is its own index - no round trip to the launch's counter before it can start.  Not when launches overlap: CTAs then
-    // trickle in as their predecessors' retire, and a pair pinned to a late CTA would hold up everything behind it.
-    bool first_pair = p.sched_check == 0;
+    bool first_pair = true;
     uint32_t fed_upto = 0;  // lle_vec_parts_*: tickets below this are known to have their actions
     for (;;) {
-        uint32_t pair = warp_global;
-        if (!first_pair) {
-            if (lane == 0) {
-                if (chunk_next >= chunk_end) {
-                    chunk_next = (p.sched_check == 0 ? p.n_warps_total : 0u) + atomicAdd(&p.sched[0], chunk);  // behind the static pairs, if any
-                    chunk_end = chunk_next + chunk;
-                }
-                pair = chunk_next++;
-            }
-            pair = __shfl_sync(kFull, pair, 0);
-        }
+        uint32_t pair = 0;
+        if (lane == 0) pair = take_pair(p, first_pair, warp_global);
+        pair = __shfl_sync(kFull, pair, 0);
         first_pair = false;
         if (pair >= n_pairs) break;
         const uint32_t ticket = single_step ? pair : pair % p.n_tickets;
