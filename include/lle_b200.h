@@ -501,6 +501,31 @@ LLE_API int lle_gen_geometry_valid(const uint8_t* cells_host, int32_t height, in
  * needed (without the terminator) in *len; writes at most cap bytes including the terminator. */
 LLE_API int lle_gen_cells_to_text(const uint8_t* cells_host, int32_t height, int32_t width, char* out, size_t cap, size_t* len);
 
+/* =====================================================================================================================
+ * Planner: exact shortest death-free joint plans, one map per CTA (breadth-first search over joint states on the device).
+ *
+ * From World::reset, every joint action of the product of the agents' available actions is stepped by the engine's own
+ * rules; a successor in which an agent died is dropped.  A goal is a state where every agent has arrived (n_arrived ==
+ * n_agents) and, with LLE_PLAN_ALL_GEMS, every gem is collected.  A state where every agent has arrived is not expanded.
+ *   length[m]      length of the shortest plan of map m: 0 when the reset state is a goal, -1 when there is none within
+ *                  max_steps steps (or when the reachable states run out first)
+ *   n_states[m]    distinct joint states reached, the reset state included, until the search stopped: at the end of the
+ *                  depth of the first goal, when no new state was reached, or after max_steps depths
+ *   actions        i8[n_maps][max_steps][4]: row t of map m is the joint action of step t (Action values, agent a in
+ *                  column a); rows from length[m] on and columns from n_agents on are -1
+ * State key: each agent's cell as an index among the map's standable cells (not wall, not laser source, not void), in mixed
+ * radix (agent 0 least significant); with LLE_PLAN_ALL_GEMS the collected-gem mask is the most significant digit.  The plan
+ * is unique: it ends in the goal state of smallest key, and the parent of a state first reached at depth d+1 is the
+ * predecessor at depth d with the smallest (parent key, joint action index), joint action index = sum_a act[a] * 5^a.
+ * Limits (LLE_LIMIT_EXCEEDED, the message names the map): n_agents <= 4; an engine record of at most 8 words with one
+ * word per beam (beams <= 32 cells) and at most 32 gems; n_cells^n_agents (times 2^n_gems with LLE_PLAN_ALL_GEMS) <= 2^22.
+ * Maps with random start candidates and max_steps outside [1, 1024] are LLE_INVALID_ARGUMENT.  Every argument and map is
+ * checked before any device call.  The buffers are host memory; the call is synchronous.  The maps may differ in shape.
+ * ===================================================================================================================== */
+enum { LLE_PLAN_ALL_GEMS = 1 };
+LLE_API int lle_plan(const lle_map* const* maps, int32_t n_maps, int32_t max_steps, uint32_t flags, int32_t device, int32_t* length,
+                     int64_t* n_states, int8_t* actions);
+
 #ifdef __cplusplus
 }
 #endif

@@ -14,6 +14,7 @@
 #include "../../include/lle_b200.h"
 #include "levels_embedded.inc"
 #include "map_compiler.hpp"
+#include "plan_core.cuh"
 #include "world_kernel.cuh"
 #include "tiny_kernel.cuh"
 
@@ -524,6 +525,17 @@ int lle_map_lasers(const lle_map* map, int32_t* out, int32_t cap, int32_t* n) {
 }
 
 const char* lle_map_text(const lle_map* map) { return map ? map->cm.text.c_str() : ""; }
+
+int lle_plan(const lle_map* const* maps, int32_t n_maps, int32_t max_steps, uint32_t flags, int32_t device, int32_t* length, int64_t* n_states,
+             int8_t* actions) {
+    if (n_maps > 0 && !maps) return fail(LLE_INVALID_ARGUMENT, "lle_plan: null argument");
+    std::vector<const CompiledMap*> cms;
+    for (int32_t m = 0; m < n_maps; ++m) {
+        if (!maps[m]) return fail(LLE_INVALID_ARGUMENT, "lle_plan: map " + std::to_string(m) + " is null");
+        cms.push_back(&maps[m]->cm);
+    }
+    return plan_run(cms.data(), n_maps, max_steps, flags, device, length, n_states, actions);
+}
 
 void lle_vec_default_options(lle_vec_options* o) {
     std::memset(o, 0, sizeof *o);

@@ -172,8 +172,10 @@ class WorldGenerator:
 
 class GeneratorBuilder:
     """lle.generate(...) (builder.py:59-437): the fluent description of a generation request.  The behavioural methods of
-    the reference (`cooperative()`, `sequential()` ...) need its SAT characterizer and raise here; `walkable()`,
-    `independent_paths()` and `needs_blocker()` select this library's reachability labels instead."""
+    the reference (`solvable()`, `cooperative()`, `sequential()` ...) need its SAT characterizer and raise here: they are
+    the reference's SAT semantics, whose encoding forbids agents following each other and swapping places
+    (world_filter.py), which this engine allows.  `walkable()`, `independent_paths()` and `needs_blocker()` select this
+    library's reachability labels instead, and `plannable(max_steps)` keeps the layouts the device planner can finish."""
 
     def __init__(self, *, width: int = 10, height: int = 10, n_agents: int = 3):
         self._kw = dict(width=width, height=height, n_agents=n_agents, starts="random", exits="random", n_gems=0, laser_placement="free",
@@ -181,6 +183,7 @@ class GeneratorBuilder:
         self._n_lasers: int | Literal["auto"] = "auto"
         self._require = 0
         self._cluster_shape = None
+        self._plan: tuple[int, bool] | None = None
 
     def random(self):
         return self.starts("random").exits("random")
@@ -243,9 +246,51 @@ class GeneratorBuilder:
         self._require = WALKABLE | NEEDS_BLOCKER
         return self
 
+    def plannable(self, max_steps: int, *, all_gems: bool = False):
+        """Keep only the layouts for which the device planner (lle_b200.planner.plan) finds a plan of at most `max_steps`
+        joint steps in which nobody dies and every agent reaches an exit (and, with `all_gems`, every gem is collected).
+        Applied after the other filters; `take` keeps the attempt order, and `build` returns the first such layout of the
+        same attempt-ordered stream.  Layouts the map compiler refuses are dropped; a layout beyond the planner's limits
+        (include/lle_b200.h: lle_plan) raises."""
+        if not 1 <= int(max_steps) <= 1024:
+            raise ValueError(f"max_steps must be in [1, 1024], got {max_steps}")
+        self._plan = (int(max_steps), bool(all_gems))
+        return self
+
+    def _plannable(self, texts: Iterator[str], n: int, device: int) -> Iterator[str]:
+        """The texts of `texts` that have a plan, in order, planned in batches of up to 1,024 maps, until n are found."""
+        from .planner import plan
+        from .types import ParsingError
+        from .vec_world import Map
+
+        max_steps, all_gems = self._plan
+        found, batch = 0, []
+        if n <= 0:
+            return
+
+        def flush():
+            length = plan(batch, max_steps=max_steps, all_gems=all_gems, device=device).length
+            return [m.text for m, k in zip(batch, length) if k >= 0]
+
+        for text in texts:
+            try:
+                batch.append(Map(text))
+            except ParsingError:
+                continue
+            if len(batch) < min(1024, 2 * (n - found)):
+                continue
+            for kept in flush():
+                yield kept
+                found += 1
+                if found == n:
+                    return
+            batch = []
+        for kept in flush()[: n - found] if batch else []:
+            yield kept
+
     def _sat_only(self, *_a, **_k):
         raise NotImplementedError("this predicate needs the reference's SAT characterizer (world_filter.py), which is out of scope; "
-                                  "use walkable() / independent_paths() / needs_blocker() (reachability labels)")
+                                  "use walkable() / independent_paths() / needs_blocker() (reachability labels) or plannable(max_steps) (device planner)")
 
     solvable = independent = cooperative = sequential = mutual = interdependent = convergent = divergent = asymmetric = require = _sat_only
 
@@ -254,10 +299,14 @@ class GeneratorBuilder:
         return WorldGenerator(**self._kw, n_lasers=n_lasers, require=self._require, cluster_shape=self._cluster_shape, device=device, batch=batch)
 
     def build(self, *, seed: int | None = None, max_attempts: int | None = None, device: int = 0):
-        """One `World` (builder.py:321-344, the n_jobs=1 path: one stream across the attempts)."""
+        """One `World` (builder.py:321-344, the n_jobs=1 path: one stream across the attempts; with `plannable`, the first
+        plannable layout of `take`'s attempt-ordered stream)."""
         from .world import World
 
-        text = self._make_generator(device, batch=1).generate(max_attempts, seed)
+        if self._plan is not None:
+            text = next(iter(self.take(1, seed=seed, max_attempts=max_attempts, device=device, texts=True)), None)
+        else:
+            text = self._make_generator(device, batch=1).generate(max_attempts, seed)
         return None if text is None else World(text)
 
     def take(self, n: int, *, seed: int | None = None, max_attempts: int | None = None, device: int = 0, distinct: bool = False,
@@ -266,7 +315,11 @@ class GeneratorBuilder:
         `texts=True` the v1 map texts instead, which is what a batch wants (`VecWorld(list_of_texts, ...)`)."""
         from .world import World
 
-        for text in self._make_generator(device).generate_n(n, seed=seed, max_attempts=max_attempts, distinct=distinct):
+        stream = self._make_generator(device).generate_n(n if self._plan is None else sys.maxsize, seed=seed, max_attempts=max_attempts,
+                                                         distinct=distinct)
+        if self._plan is not None:
+            stream = self._plannable(stream, n, device)
+        for text in stream:
             yield text if texts else World(text, device)
 
 
