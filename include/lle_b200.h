@@ -526,6 +526,41 @@ enum { LLE_PLAN_ALL_GEMS = 1 };
 LLE_API int lle_plan(const lle_map* const* maps, int32_t n_maps, int32_t max_steps, uint32_t flags, int32_t device, int32_t* length,
                      int64_t* n_states, int8_t* actions);
 
+/* =====================================================================================================================
+ * Expert: exact distance-to-goal tables for the maps of a vec, and the optimal joint action of every world of it.
+ *
+ * State, key, step, goal and limits are lle_plan's: the key is each agent's index among the standable cells in mixed radix
+ * (with LLE_PLAN_ALL_GEMS the collected-gem mask is the top digit); successors come from every available joint action stepped
+ * by the engine, and a successor in which an agent died is dropped; a goal is n_arrived == n_agents (and every gem with
+ * LLE_PLAN_ALL_GEMS); a state where every agent has arrived is not expanded.  Limits (LLE_LIMIT_EXCEEDED, naming the map):
+ * n_agents <= 4, an engine record of at most 8 words with one word per beam and at most 32 gems, K = n_cells^n_agents
+ * (x 2^n_gems with LLE_PLAN_ALL_GEMS) <= 2^22; maps with random starts are LLE_INVALID_ARGUMENT.
+ *   reached set  every state reachable from the map's reset state through death-free transitions, with no depth cap (the
+ *                enumeration does not stop at the first goal); the reset state is included.
+ *   dist(s)      the length of a shortest death-free path from s to a goal: 0 on a goal, "none" when no reached successor chain
+ *                ends in a goal (an all-arrived state missing gems under LLE_PLAN_ALL_GEMS included).  32-bit, no saturation.
+ *   joint(s)     for dist(s) > 0, the smallest joint action index j = sum_a act[a] * 5^a whose every act[a] is available (the
+ *                record's availability cache), with which nobody dies, and whose successor has dist(s) - 1.
+ * The tables are therefore unique: every build of the same maps gives the same bytes, whatever the schedule.
+ * The vec must have walkable_lasers = 1 (otherwise its availability mask is not the engine's) and no randomize_lasers; no
+ * pipelined or parts-loop step may be outstanding.  All of these, null arguments and unknown flags are LLE_INVALID_ARGUMENT,
+ * checked before any device work; so is act / table before a build, or after a set_source / set_exits that followed it (a
+ * change of the map drops its vec's tables; collect_gem does not change the dynamics and keeps them).
+ * ===================================================================================================================== */
+/* Builds the tables of the vec's maps as the vec holds them now (after lle_vec_set_source / set_exits), on the device.
+ * n_states: host i64[n_maps] or NULL, the size of each map's reached set.  LLE_LIMIT_EXCEEDED when a map is over the limits
+ * or when the tables and the build's state array (up to sum K entries) do not fit the free device memory.  Synchronous. */
+LLE_API int lle_vec_expert_build(lle_vec* vec, uint32_t flags /* LLE_PLAN_ALL_GEMS */, int64_t* n_states, void* cuda_stream);
+/* Per env, from its current engine record, asynchronous on cuda_stream (an ordinary launch, ordered after the step before it):
+ *   actions_dev i8[N, A]: joint(s) when dist > 0, else Stay (4) for every agent; directly usable as lle_vec_step's actions_dev
+ *   dist_dev    i32[N] or NULL: dist(s) >= 0; -1 reached but no death-free way to a goal;
+ *               -2 not in the table (an agent is dead, or the state is not reachable from reset without a death, e.g. after
+ *               lle_vec_set_state) */
+LLE_API int lle_vec_expert_act(lle_vec* vec, int8_t* actions_dev, int32_t* dist_dev, void* cuda_stream);
+/* Host copy of map m's table: dist i32[K] (-2 not reached, -1 none, >= 0) and joint i16[K] (-1 where dist <= 0 or not reached);
+ * either may be NULL.  *n_keys receives K; copies min(K, cap) entries. */
+LLE_API int lle_vec_expert_table(lle_vec* vec, int32_t map_index, int32_t* dist_host, int16_t* joint_host, int64_t cap, int64_t* n_keys);
+
 #ifdef __cplusplus
 }
 #endif

@@ -26,6 +26,7 @@ SYMBOLS = [
     "lle_vec_parts_end", "lle_vec_parts_abort",
     "lle_gen_default_options", "lle_gen_create", "lle_gen_destroy", "lle_gen_attempt_seeds", "lle_gen_run", "lle_gen_get_buffers",
     "lle_gen_fetch", "lle_gen_geometry_valid", "lle_gen_cells_to_text", "lle_plan",
+    "lle_vec_expert_build", "lle_vec_expert_act", "lle_vec_expert_table",
 ]
 
 
@@ -152,6 +153,9 @@ def lib():
     L.lle_gen_geometry_valid.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]
     L.lle_gen_cells_to_text.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]
     L.lle_plan.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_uint32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.lle_vec_expert_build.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
+    L.lle_vec_expert_act.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.lle_vec_expert_table.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]
     _lib = L
     return L
 

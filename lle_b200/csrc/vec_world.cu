@@ -14,7 +14,7 @@
 #include "../../include/lle_b200.h"
 #include "levels_embedded.inc"
 #include "map_compiler.hpp"
-#include "plan_core.cuh"
+#include "expert_core.cuh"
 #include "world_kernel.cuh"
 #include "tiny_kernel.cuh"
 
@@ -147,6 +147,8 @@ struct lle_vec {
     const void* pinned_seen[32] = {};  // host pointers already checked to be page-locked ...
     void* pinned_dev[32] = {};         // ... and the address the device reaches them at
     unsigned pinned_next = 0;
+    // lle_vec_expert_build: the distance tables of the maps as they were at the build (dropped by swap_map)
+    ExpertTables* expert = nullptr;
 };
 
 namespace {
@@ -551,6 +553,7 @@ int lle_vec_destroy(lle_vec* v) {
     cudaSetDevice(v->device);
     if (v->parts_n) lle_vec_parts_abort(v);  // no kernel may be left waiting for actions
     if (v->shadow) lle_vec_destroy(v->shadow);
+    expert_free(v->expert);
     if (v->borrows_records) { v->d_records = nullptr; v->d_map_of_env = nullptr; }
     for (auto* b : v->d_blobs) cudaFree(b);
     for (auto* b : v->retired_blobs) cudaFree(b);
@@ -984,6 +987,8 @@ int swap_map(lle_vec* v, int map_index, const std::vector<SourceState>& sources,
         v->map0 = host_bind(d, cm.header());
     }
     v->last_was_step = false;
+    expert_free(v->expert);  // the dynamics of the map may have changed: the tables no longer describe it
+    v->expert = nullptr;
     if (out_cm) *out_cm = std::move(cm);
     return LLE_OK;
 }
@@ -1503,6 +1508,68 @@ int lle_vec_set_seed(lle_vec* v, uint64_t seed) { if (!v) return fail(LLE_INVALI
 int lle_vec_get_step_count(lle_vec* v, uint64_t* out) { if (!v || !out) return fail(LLE_INVALID_ARGUMENT, "null"); *out = v->t; return LLE_OK; }
 int lle_vec_set_step_count(lle_vec* v, uint64_t value) { if (!v) return fail(LLE_INVALID_ARGUMENT, "null"); v->t = value; return LLE_OK; }
 int lle_vec_launch_count(lle_vec* v, uint64_t* out) { if (!v || !out) return fail(LLE_INVALID_ARGUMENT, "null"); *out = v->launches; return LLE_OK; }
+
+// ---- the device expert (include/lle_b200.h; the tables and kernels are expert.cu's)
+namespace {
+const char* const kOutstanding =
+    "pipelined steps outstanding: drain with lle_vec_pipeline_wait (or close the parts loop with lle_vec_parts_end) first";
+ExpertVecView expert_view(const lle_vec* v) {
+    ExpertVecView e;
+    e.device = v->device;
+    e.N = v->N;
+    e.A = v->A; e.G = v->G; e.W = v->W;
+    e.L = v->L;
+    e.records = v->d_records;
+    e.map_of_env = v->d_map_of_env;
+    return e;
+}
+}  // namespace
+
+int lle_vec_expert_build(lle_vec* v, uint32_t flags, int64_t* n_states, void* stream) {
+    if (!v) return fail(LLE_INVALID_ARGUMENT, "null vec");
+    if (flags & ~(uint32_t)LLE_PLAN_ALL_GEMS) return fail(LLE_INVALID_ARGUMENT, "lle_vec_expert_build: unknown flag");
+    if (!v->opts.walkable_lasers)
+        return fail(LLE_INVALID_ARGUMENT, "lle_vec_expert_build: walkable_lasers = 0 (the env's availability mask is not the engine's)");
+    if (v->randomize) return fail(LLE_INVALID_ARGUMENT, "lle_vec_expert_build: not with randomize_lasers");
+    if (v->pipe_submitted != v->pipe_completed || v->parts_n) return fail(LLE_INVALID_ARGUMENT, kOutstanding);
+    // the maps as the vec steps them now: recompiled like swap_map does, with the current sources and exits
+    std::vector<CompiledMap> cms;
+    try {
+        for (size_t m = 0; m < v->map_texts.size(); ++m)
+            cms.push_back(compile_map(v->map_texts[m], ObsSpec{v->opts.obs_type, v->opts.obs_param, v->opts.obs_dtype}, &v->src_state[m],
+                                      v->map_exits_set[m] ? &v->map_exits[m] : nullptr));
+    } catch (const MapError& e) {
+        return fail(e.status, e.what());
+    }
+    ExpertVecView view = expert_view(v);
+    for (size_t m = 0; m < cms.size(); ++m) {
+        view.maps.push_back(&cms[m]);
+        view.blobs.push_back(v->d_blobs[m]);
+    }
+    ExpertTables* t = nullptr;
+    if (int rc = expert_build(view, flags, n_states, stream, &t)) return rc;
+    expert_free(v->expert);
+    v->expert = t;
+    return LLE_OK;
+}
+
+int lle_vec_expert_act(lle_vec* v, int8_t* actions_dev, int32_t* dist_dev, void* stream) {
+    if (!v || !actions_dev) return fail(LLE_INVALID_ARGUMENT, "null argument");
+    if (!v->expert) return fail(LLE_INVALID_ARGUMENT, "lle_vec_expert_act: no tables (call lle_vec_expert_build, again after set_source / set_exits)");
+    if (v->pipe_submitted != v->pipe_completed || v->parts_n) return fail(LLE_INVALID_ARGUMENT, kOutstanding);
+    if (int rc = expert_act(expert_view(v), v->expert, actions_dev, dist_dev, stream)) return rc;
+    v->last_was_step = false;  // an ordinary launch: the next step must not overlap it
+    v->launches++;
+    return LLE_OK;
+}
+
+int lle_vec_expert_table(lle_vec* v, int32_t map_index, int32_t* dist_host, int16_t* joint_host, int64_t cap, int64_t* n_keys) {
+    if (!v || !n_keys || cap < 0) return fail(LLE_INVALID_ARGUMENT, "bad argument");
+    if (map_index < 0 || map_index >= (int)v->map_texts.size()) return fail(LLE_INVALID_ARGUMENT, "map index out of range");
+    if (!v->expert) return fail(LLE_INVALID_ARGUMENT, "lle_vec_expert_table: no tables (call lle_vec_expert_build, again after set_source / set_exits)");
+    if (v->pipe_submitted != v->pipe_completed || v->parts_n) return fail(LLE_INVALID_ARGUMENT, kOutstanding);
+    return expert_table(v->expert, map_index, dist_host, joint_host, cap, n_keys);
+}
 
 int lle_vec_timing_begin(lle_vec* v, void* stream) {
     if (!v) return fail(LLE_INVALID_ARGUMENT, "null vec");

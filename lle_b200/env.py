@@ -8,6 +8,7 @@ from __future__ import annotations
 
 from typing import Sequence
 
+import numpy as np
 import torch
 
 from .types import obs_spec
@@ -69,6 +70,14 @@ class VecLLE:
         """actions: int8 (N, A) on the device, or None to sample uniformly among available actions on the GPU."""
         self.world.step(actions)
         return self.obs, self.state, self.reward, self.done
+
+    def build_expert(self, all_gems: bool = False) -> np.ndarray:
+        """Distance-to-goal tables of the maps (VecWorld.build_expert): the size of each map's reached set."""
+        return self.world.build_expert(all_gems)
+
+    def expert_actions(self, actions_out: torch.Tensor | None = None, dist_out: torch.Tensor | None = None):
+        """The optimal joint action of every env and its distance to a goal (VecWorld.expert_actions)."""
+        return self.world.expert_actions(actions_out, dist_out)
 
     def dlpack(self, name: str):
         return getattr(self, name).__dlpack__()

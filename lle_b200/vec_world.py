@@ -399,6 +399,42 @@ class VecWorld:
         check(lib().lle_vec_set_state(self._h, pos.data_ptr(), gems.data_ptr() if self.n_gems else None, alive.data_ptr(),
                                       _stream_ptr(self.device)))
 
+    # ---- the device expert (include/lle_b200.h: lle_vec_expert_*)
+    def build_expert(self, all_gems: bool = False) -> np.ndarray:
+        """Builds, on the device, the exact distance-to-goal table of every map as the batch holds it now: over every joint state
+        reachable from reset without a death, the length of a shortest death-free way to a goal (every agent on an exit, and with
+        `all_gems` every gem collected) and the smallest joint action that starts one.  Returns the size of each map's reached set
+        (int64 [n_maps]).  Limits: those of `lle_b200.planner.plan`; the batch needs walkable_lasers and no randomize_lasers.
+        `set_source` / `set_exits` drop the tables: build again after them."""
+        n_states = np.zeros(len(self.maps), np.int64)
+        check(lib().lle_vec_expert_build(self._h, 1 if all_gems else 0, n_states.ctypes.data_as(C.c_void_p), _stream_ptr(self.device)))
+        return n_states
+
+    def expert_actions(self, actions_out: torch.Tensor | None = None, dist_out: torch.Tensor | None = None):
+        """(actions int8 [N, A], dist int32 [N]) of every env from its current state, on the batch's device and torch's current
+        stream: the optimal joint action (all Stay where dist <= 0), directly usable as `step`'s actions, and the distance to a goal
+        (-1: no death-free way there; -2: not in the table, an agent is dead or the state is not reachable from reset)."""
+        N, A = self.n_envs, self.n_agents
+        if actions_out is None:
+            actions_out = torch.empty((N, A), dtype=torch.int8, device=self.device)
+        if dist_out is None:
+            dist_out = torch.empty((N,), dtype=torch.int32, device=self.device)
+        for t, dt, shape in ((actions_out, torch.int8, (N, A)), (dist_out, torch.int32, (N,))):
+            if t.dtype != dt or tuple(t.shape) != shape or t.device != self.device or not t.is_contiguous():
+                raise ValueError(f"expert_actions: expected a contiguous {dt} {shape} tensor on {self.device}")
+        check(lib().lle_vec_expert_act(self._h, actions_out.data_ptr(), dist_out.data_ptr(), _stream_ptr(self.device)))
+        return actions_out, dist_out
+
+    def expert_table(self, map_index: int = 0) -> tuple[np.ndarray, np.ndarray]:
+        """Host copy of map `map_index`'s table, indexed by state key (include/lle_b200.h: lle_vec_expert_build): dist int32 [K]
+        (-2 not reached, -1 no way to a goal, else the distance) and joint int16 [K] (sum_a act[a] * 5^a; -1 where dist <= 0)."""
+        K = C.c_int64(0)
+        check(lib().lle_vec_expert_table(self._h, int(map_index), None, None, 0, C.byref(K)))
+        dist, joint = np.zeros(K.value, np.int32), np.zeros(K.value, np.int16)
+        check(lib().lle_vec_expert_table(self._h, int(map_index), dist.ctypes.data_as(C.c_void_p), joint.ctypes.data_as(C.c_void_p),
+                                         K.value, C.byref(K)))
+        return dist, joint
+
     def export_raw(self) -> dict[str, torch.Tensor]:
         N, A, NB = self.n_envs, self.n_agents, max(self.n_beams_max, 1)
         d = self.device
